@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the cnf_ot flow train step (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--reps R] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--reps R] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" = one evaluation of the configured MFC loss and its parameter gradient
 (all flow passes forward + inverse + log-det + loss terms + backward; optimiser
@@ -10,7 +10,11 @@ configs[1]: mfc.yaml type=ot subtype=obstacle, 2-D, RQS flow (2 layers, 2x16
 conditioner, 5 bins), batch 2^18 per GPU (weak scaling), lambda=5000, dt=0.01.
 
   value       samples/s with the batch already resident in HBM (CUDA events, max over ranks;
-              median of --reps repetitions of the K-step block, min / max in `spread`)
+              K timed steps split into --reps blocks, median of the blocks, min / max in `spread`)
+  --dump-outputs DIR : [gradient | loss slots] of the last timed step (headline workload, or the --only
+              config) as DIR/gradient.npy and DIR/loss_slots.npy (float32); seeded inputs, so two builds
+              compare output for output.  At most 64 MiB: a larger gradient is written as a fixed, seeded
+              sample of 2^20 entries, their indices in DIR/gradient_index.npy
   e2e         the same through the C-ABI call with HOST (pinned) buffers: H2D of the inputs
               and the weights, the step, D2H of [gradient | loss] inside the timed region
   parity      the SAME parameter blob and the SAME 2^18-row input set evaluated by the CPU
@@ -357,11 +361,22 @@ class Dist:
 
 
 def timed_reps(dist, step, steps, reps):
-  """`reps` repetitions of a `steps`-step block; per-step seconds of each block, max over ranks."""
-  per = []
-  for r in range(reps):
-    per.append(time_region(step, steps, dist.sync, first=r * steps) / steps)
-  return dist.max_over_ranks(per)
+  """`steps` consecutive timed steps (indices 0 .. steps-1) in `reps` blocks (fewer when steps < reps); per-step
+  seconds of each block, max over ranks.  The blocks are delimited by events recorded between the steps, with no
+  synchronise between them, so only the first block starts from an idle device."""
+  reps = max(1, min(reps, steps))
+  sizes = [steps // reps + (r < steps % reps) for r in range(reps)]
+  ev = [torch.cuda.Event(enable_timing=True) for _ in range(reps + 1)]
+  dist.sync()
+  ev[0].record()
+  i = 0
+  for r, n in enumerate(sizes):
+    for _ in range(n):
+      step(i)
+      i += 1
+    ev[r + 1].record()
+  dist.sync()
+  return dist.max_over_ranks([ev[r].elapsed_time(ev[r + 1]) / 1e3 / n for r, n in enumerate(sizes)])
 
 
 def spread(per_step_s):
@@ -692,7 +707,7 @@ def density_block(dev):
 
 def per_config_entry(name, dist, args, pk, pk_src):
   """Timing + roofline + small-batch oracle check of one BASELINE config other than the headline one."""
-  steps = {"cfg1": 50, "cfg2": 20, "cfg3": 10, "cfg4": 3, "cfg5": 2}[name]
+  steps = {"cfg1": 250, "cfg2": 100, "cfg3": 50, "cfg4": 9, "cfg5": 2}[name]
   reps = {"cfg1": 5, "cfg2": 5, "cfg3": 5, "cfg4": 3, "cfg5": 1}[name]
   if args.only:
     steps, reps = args.steps, args.reps
@@ -701,6 +716,8 @@ def per_config_entry(name, dist, args, pk, pk_src):
   for i in range(3 if name != "cfg5" else 1):
     w.step(i)
   per = timed_reps(dist, w.step, steps, reps)
+  if args.only and args.dump_outputs and dist.rank == 0:
+    dump_outputs(args.dump_outputs, w.shape, w.out)
   t_step = statistics.median(per)
   entry = {
     "workload": w.label, "dim": w.D, "params": w.shape.blob_size, "batch_per_gpu": w.B, "global_batch": w.gB,
@@ -726,6 +743,28 @@ def per_config_entry(name, dist, args, pk, pk_src):
       entry["oracle_check"] = {"error": repr(exc)}
     torch.cuda.empty_cache()
   return entry
+
+
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SAMPLE = 1 << 20
+
+
+def dump_outputs(path, shape, out):
+  """The buffer the last timed step returned to its caller, [gradient | loss slots] (include/cnfot.h), as
+  path/gradient.npy and path/loss_slots.npy (float32): the inputs are seeded, so two builds compare output for output.
+  A buffer over DUMP_MAX_BYTES (cfg 5: 139 M parameters) keeps the files under it: gradient.npy then holds the entries
+  at DUMP_SAMPLE indices drawn without replacement from a fixed seed, written in ascending order to
+  gradient_index.npy (float64, exact)."""
+  import numpy as np
+  os.makedirs(path, exist_ok=True)
+  n = shape.blob_size
+  grad = out.detach()[:n]
+  if out.numel() * 4 > DUMP_MAX_BYTES:
+    idx = np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLE, replace=False))
+    grad = grad[torch.from_numpy(idx).to(grad.device)]
+    np.save(os.path.join(path, "gradient_index.npy"), idx.astype(np.float64))
+  np.save(os.path.join(path, "gradient.npy"), grad.float().cpu().numpy())
+  np.save(os.path.join(path, "loss_slots.npy"), out.detach()[n:].float().cpu().numpy())
 
 
 def timeline_block(w, n=24):
@@ -775,6 +814,8 @@ def run_ours(args):
   value = w.gB / t_step
   loss_dev = float(w.out[n])
   launch = _lib.last_launch_info()
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, shape, w.out)
 
   # ---- parity at the FULL batch: same blob, same input set, CPU oracle (rank 0's shard as a whole batch)
   parity = None
@@ -895,7 +936,7 @@ def run_ours(args):
                                      "api": "cnfot_mfc_step_host: pinned host row arrays read in place over PCIe (round-1 form)"}},
       "on_chip_draws": {"value": w.gB / t_rng, "ms_per_step": t_rng * 1e3,
                         "note": "cnfot_mfc_step_rng, device-timed: same step, rows generated in the kernel instead of read from HBM"},
-      "gpu_launches": args.steps * args.reps,  # ONE kernel per step: mfc_step_kernel (reduction, all-reduce in its tail)
+      "gpu_launches": args.steps,  # ONE kernel per step: mfc_step_kernel (reduction, all-reduce in its tail)
       "clocks": clk.summary(),
       "parity": parity, "dp_check": dp_check,
       "step_timeline": timeline,
@@ -961,15 +1002,24 @@ def run_only(args):
 def main():
   ap = argparse.ArgumentParser()
   ap.add_argument("--gpus", type=int, default=1)
-  ap.add_argument("--steps", type=int, default=20)
+  ap.add_argument("--steps", type=int, default=None, help="timed steps K (default 100; 20 for --impl reference)")
   ap.add_argument("--warmup", type=int, default=5)
-  ap.add_argument("--reps", type=int, default=5, help="repetitions of the K-step timed block (median reported)")
+  ap.add_argument("--reps", type=int, default=5, help="blocks the K timed steps are split into (median reported)")
   ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
   ap.add_argument("--no-per-config", action="store_true", help="skip the per_config block (configs 1, 3, 4, 5)")
   ap.add_argument("--no-oracle", action="store_true", help="skip every CPU-oracle leg (parity, cpu_baseline)")
   ap.add_argument("--only", default=None, choices=sorted(WORKLOADS), help="time ONE config alone (builder tool)")
   ap.add_argument("--rows-per-gpu", type=int, default=None, help="--only: rows per GPU (weak scaling)")
+  ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                  help="write what the last timed step returned as DIR/<name>.npy, at most 64 MiB (a larger "
+                       "gradient as a seeded sample); not with --impl reference")
   args = ap.parse_args()
+  if args.steps is None:
+    args.steps = 20 if args.impl == "reference" else 100
+  if args.steps < 1:
+    ap.error("--steps must be at least 1")
+  if args.dump_outputs and args.impl == "reference":
+    ap.error("--dump-outputs: the reference arm sizes its row sample from a timing probe, so its inputs differ from run to run")
   if args.impl == "reference":
     run_reference(args)
   elif args.only:

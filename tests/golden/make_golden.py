@@ -1,6 +1,7 @@
 """Generate the golden fixtures under tests/golden/ from the CPU oracle (torch float64).
 
   python tests/golden/make_golden.py
+  python -c "import make_golden; make_golden.save_mirror_signatures()"   (from tests/golden: the API record alone)
 
 PROVENANCE: these vectors are outputs of oracle/ (the restatement of the reference), NOT of the reference itself; the
 fixtures produced by the reference's own code are tests/golden/ref_*.npz (make_reference_golden.py), which also pin
@@ -102,6 +103,31 @@ def save(name, d):
   print(name, {k: v.shape for k, v in out.items()})
 
 
+# the mirror's API that tests/test_reference_golden.py compares with the original project's source
+# (None: every public function of the module)
+SIGNATURES = {"cnf_ot_b200.applications": None,
+              "cnf_ot_b200.utils": ["calc_kinetic_energy", "calc_score_kinetic_energy"],
+              "cnf_ot_b200.flows": ["RQSFlow"], "cnf_ot_b200.solvers": ["main"]}
+
+
+def save_mirror_signatures():
+  """mirror_signatures.json: parameter names of the mirror's API as this repository defines it (NOT read from the
+  original project), so that the mirror cannot drift without a test failing where the original is not at hand."""
+  import importlib
+  import inspect
+  import json
+  out = {}
+  for mod_name, names in SIGNATURES.items():
+    mod = importlib.import_module(mod_name)
+    if names is None:
+      names = sorted(n for n, f in inspect.getmembers(mod, inspect.isfunction)
+                     if f.__module__ == mod_name and not n.startswith("_"))
+    out[mod_name] = {n: list(inspect.signature(getattr(mod, n)).parameters) for n in names}
+  with open(os.path.join(HERE, "mirror_signatures.json"), "w") as f:
+    json.dump(out, f, indent=1)
+    f.write("\n")
+
+
 STEP_CASES = {
   # hidden 64: outside the fused kernels, runs on the wide-conditioner engine (csrc/wide.cu)
   "step_ot_free_d3_h64": ("ot", "free", 256, 500.0, 2, dict(dim=3, H=64, sigma=0.05)),
@@ -120,3 +146,4 @@ if __name__ == "__main__":
   save("dr_dec_only_d4", dr_case("dec_only", 4, 2, 16, 2, 0.08, 320, 13))
   for name, (typ, sub, B, lam, Tn, kw) in STEP_CASES.items():
     save(name, step_case(typ, sub, B, lam, Tn, **dict(kw)))
+  save_mirror_signatures()

@@ -1,9 +1,10 @@
 """Execute the reference's OWN unit test of the spline, unmodified, against the stand-in spline (oracle/rqs.py behind the
 `distrax.RationalQuadraticSpline` interface of tests/golden/refshim.py):
 
-  python tests/golden/run_reference_tests.py         (needs /root/reference; exit code 0 = every test method passed)
+  CNF_OT_REFERENCE=<checkout of the original cnf_ot project> python tests/golden/run_reference_tests.py
+                                                     (exit code 0 = every test method passed)
 
-/root/reference/tests/test_rqs_accuracy.py holds the reference's known-answer checks for this path (SURVEY.md section 8c):
+The original project's tests/test_rqs_accuracy.py holds the reference's known-answer checks for this path (SURVEY.md section 8c):
 forward-inverse and inverse-forward round trips, log-det against the autodiff Jacobian, boundary round trips, all < 1e-12
 in float64 on three spline configurations.  Run in its own process: the stand-ins register fake `jax` / `distrax` modules.
 """
@@ -22,7 +23,9 @@ import refshim  # noqa: E402
 refshim.install()
 refshim.Draws.set()   # nothing programmed: jax.random.uniform is a seeded stream per key
 
-path = "/root/reference/tests/test_rqs_accuracy.py"
+if not os.environ.get("CNF_OT_REFERENCE"):
+  sys.exit("set CNF_OT_REFERENCE to a checkout of the original cnf_ot project")
+path = os.path.join(os.environ["CNF_OT_REFERENCE"], "tests", "test_rqs_accuracy.py")
 spec = importlib.util.spec_from_file_location("reference_test_rqs_accuracy", path)
 mod = importlib.util.module_from_spec(spec)
 spec.loader.exec_module(mod)

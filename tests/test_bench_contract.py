@@ -27,6 +27,67 @@ def test_reference_arm_prints_one_json_line():
   assert "workload" in d["config"] and "model" not in d["config"]
 
 
+@pytest.mark.gpu
+def test_bench_times_k_steps_and_dumps_the_last_one(tmp_path):
+  """--steps K times steps 0 .. K-1 however many blocks --reps splits them into, and --dump-outputs writes the
+  [gradient | loss slots] buffer the last of them returned.  Step i reads its own seeded input set and time, so the dump
+  tells which step ran last: runs that end on the same step agree, a run one step longer does not."""
+  import numpy as np
+
+  def run(out, *args):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--warmup", "1", "--no-oracle",
+                        "--dump-outputs", str(out), *args], capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-2000:]
+    g, s = np.load(out / "gradient.npy"), np.load(out / "loss_slots.npy")
+    assert g.dtype == s.dtype == np.float32 and s.shape == (8, ) and np.isfinite(g).all()
+    return json.loads(r.stdout), np.concatenate([g, s]).astype(np.float64)
+
+  def headline(steps, reps):
+    d, v = run(tmp_path / f"k{steps}_r{reps}", "--steps", str(steps), "--reps", str(reps), "--no-per-config")
+    assert d["steps"] == steps and d["spread"]["reps"] == min(steps, reps) and v.size == d["config"]["params"] + 8
+    assert v[-8] == np.float32(d["run"]["loss_last_step"])
+    return v
+
+  rel = lambda a, b: np.abs(a - b).max() / np.abs(b).max()
+  k3, k3_one_block, k4 = headline(3, 3), headline(3, 1), headline(4, 1)
+  assert rel(k3, k3_one_block) < 1e-5   # the same step: equal up to the order of the kernel's float additions
+  assert rel(k4, k3_one_block) > 1e-4   # another input set and time
+  d, v = run(tmp_path / "only", "--only", "cfg1", "--steps", "2")
+  assert v.size == d["entry"]["params"] + 8 and v[-8] == np.float32(d["entry"]["loss_last_step"])
+
+
+def test_dump_outputs_stays_within_64_mib(tmp_path):
+  """bench.dump_outputs on the CPU: a buffer within 64 MiB is written whole, a larger one (cfg 5's gradient alone is
+  530 MiB) as the same seeded sample of gradient entries every time, with their indices; all files within 64 MiB."""
+  import numpy as np
+  import torch
+  cap = 64 << 20
+  sizes = (1200, cap // 4)   # the second: [gradient | 8 loss slots] just over the cap
+  code = ("import sys, types, torch\nsys.path.insert(0, sys.argv[1])\nimport bench\n"
+          "for n in map(int, sys.argv[3:]):\n"
+          "  out = torch.rand(n + 8, generator=torch.Generator().manual_seed(n))\n"
+          "  for run in 'ab':\n"
+          "    bench.dump_outputs(f'{sys.argv[2]}/{n}{run}', types.SimpleNamespace(blob_size=n), out)\n")
+  r = subprocess.run([sys.executable, "-c", code, ROOT, str(tmp_path), *map(str, sizes)], capture_output=True, text=True,
+                     timeout=600)
+  assert r.returncode == 0, r.stderr[-2000:]
+  for n in sizes:
+    out = torch.rand(n + 8, generator=torch.Generator().manual_seed(n)).numpy()
+    d = tmp_path / f"{n}a"
+    files = {f.name: np.load(f) for f in d.iterdir()}
+    assert sum(f.stat().st_size for f in d.iterdir()) <= cap
+    assert all(v.dtype in (np.float32, np.float64) for v in files.values())
+    assert np.array_equal(files["loss_slots.npy"], out[n:])
+    if (n + 8) * 4 <= cap:
+      assert set(files) == {"gradient.npy", "loss_slots.npy"} and np.array_equal(files["gradient.npy"], out[:n])
+    else:
+      idx = files["gradient_index.npy"]
+      assert idx.size == files["gradient.npy"].size == 1 << 20 and (np.diff(idx) > 0).all() and 0 <= idx[0] <= idx[-1] < n
+      assert np.array_equal(files["gradient.npy"], out[:n][idx.astype(np.int64)])
+    for name, v in files.items():
+      assert np.array_equal(v, np.load(tmp_path / f"{n}b" / name))
+
+
 @pytest.mark.parametrize("name", ["r01_bench_n1_final.json", "r01_bench_n2_final.json", "r01_bench_n8_final.json"])
 def test_committed_bench_lines_follow_the_contract(name):
   d = json.loads(open(os.path.join(ROOT, "profiles", name)).read())

@@ -110,15 +110,29 @@ def test_oracle_ot_reverse_kl_matches_reference(name):
   assert abs(float(got) - float(g["ot_reverse_kl"])) <= 1e-12 * abs(float(g["ot_reverse_kl"]))
 
 
-REF = "/root/reference/cnf_ot"
+# a checkout of the original project (github.com/jiaxi98/cnf_ot); the two tests that read its source skip without one
+REF_ROOT = os.environ.get("CNF_OT_REFERENCE", "")
+REF = os.path.join(REF_ROOT, "cnf_ot")
+NO_REF = "needs a checkout of the original cnf_ot project in CNF_OT_REFERENCE"
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference tree only exists in the build container")
+def _check_signatures(mod, sigs, only=None):
+  """Each function of `sigs` (name -> parameter names) exists in `mod` with those parameters first, in that order;
+  any further parameters are optional."""
+  import inspect
+  for name, args in sigs.items():
+    if only is not None and name not in only:
+      continue
+    params = list(inspect.signature(getattr(mod, name)).parameters.values())
+    assert [p.name for p in params[:len(args)]] == args, (mod.__name__, name, args, params)
+    assert all(p.default is not inspect.Parameter.empty for p in params[len(args):]), (name, params[len(args):])
+
+
+@pytest.mark.skipif(not REF_ROOT or not os.path.isdir(REF), reason=NO_REF)
 def test_mirror_signatures_match_the_reference():
   """Every function of the reference's applications.py, the two energies of utils.py, RQSFlow and solvers.main exist in
   the mirror with the same parameter names in the same order (extra trailing optional parameters allowed)."""
   import ast
-  import inspect
   import cnf_ot_b200.applications as A
   import cnf_ot_b200.flows as F
   import cnf_ot_b200.solvers as S
@@ -127,22 +141,29 @@ def test_mirror_signatures_match_the_reference():
   def ref_sigs(path):
     tree = ast.parse(open(path).read())
     return {n.name: [a.arg for a in n.args.args + n.args.kwonlyargs] for n in tree.body if isinstance(n, ast.FunctionDef)}
-  checks = [(A, ref_sigs(REF + "/mfc/applications.py"), None),
-            (U, ref_sigs(REF + "/utils.py"), {"calc_kinetic_energy", "calc_score_kinetic_energy"}),
-            (F, ref_sigs(REF + "/models/flows.py"), {"RQSFlow"}), (S, ref_sigs(REF + "/mfc/solvers.py"), {"main"})]
-  for mod, sigs, only in checks:
-    for name, args in sigs.items():
-      if only is not None and name not in only:
-        continue
-      mine = list(inspect.signature(getattr(mod, name)).parameters)
-      assert mine[:len(args)] == args, (mod.__name__, name, args, mine)
-      extra = list(inspect.signature(getattr(mod, name)).parameters.values())[len(args):]
-      assert all(p.default is not inspect.Parameter.empty for p in extra), (name, extra)
+  _check_signatures(A, ref_sigs(REF + "/mfc/applications.py"))
+  _check_signatures(U, ref_sigs(REF + "/utils.py"), {"calc_kinetic_energy", "calc_score_kinetic_energy"})
+  _check_signatures(F, ref_sigs(REF + "/models/flows.py"), {"RQSFlow"})
+  _check_signatures(S, ref_sigs(REF + "/mfc/solvers.py"), {"main"})
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference tree only exists in the build container")
+def test_mirror_signatures_match_the_stored_record():
+  """The same API -- every public function of applications.py, the two energies of utils.py, RQSFlow, solvers.main --
+  against tests/golden/mirror_signatures.json (tests/golden/make_golden.py), under the same rule.  The record holds
+  the mirror's own signatures, not data read from the original project; it keeps the API from drifting where no checkout
+  of the original is at hand."""
+  import importlib
+  import json
+  with open(os.path.join(GOLD, "mirror_signatures.json")) as f:
+    record = json.load(f)
+  assert set(record) == {"cnf_ot_b200.applications", "cnf_ot_b200.utils", "cnf_ot_b200.flows", "cnf_ot_b200.solvers"}
+  for mod_name, sigs in record.items():
+    _check_signatures(importlib.import_module(mod_name), sigs)
+
+
+@pytest.mark.skipif(not REF_ROOT or not os.path.isdir(REF), reason=NO_REF)
 def test_reference_own_spline_test_passes_on_the_restated_spline():
-  """/root/reference/tests/test_rqs_accuracy.py, executed UNMODIFIED against oracle/rqs.py behind the
+  """The original project's tests/test_rqs_accuracy.py, executed UNMODIFIED against oracle/rqs.py behind the
   `distrax.RationalQuadraticSpline` interface (tests/golden/run_reference_tests.py; own process because the stand-ins
   register fake jax / distrax modules): round trips, log-det vs autodiff Jacobian, boundaries, all < 1e-12."""
   import subprocess
@@ -151,7 +172,7 @@ def test_reference_own_spline_test_passes_on_the_restated_spline():
   r = subprocess.run([sys.executable, os.path.join(here, "golden", "run_reference_tests.py")], capture_output=True,
                      text=True, timeout=600)
   assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-  assert "PASSED /root/reference/tests/test_rqs_accuracy.py::TestRQSAccuracy::test_rqs_comprehensive" in r.stdout
+  assert "PASSED " + os.path.join(REF_ROOT, "tests", "test_rqs_accuracy.py") + "::TestRQSAccuracy::test_rqs_comprehensive" in r.stdout
 
 
 @pytest.mark.parametrize("name", list(STEPS))
