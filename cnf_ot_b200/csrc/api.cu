@@ -196,7 +196,9 @@ static int make_plan(const FlowLayout& lay, bool with_grad, SmemPlan* sp, int* e
 }
 
 // Persistent launch: as many CTAs as fit on the chip, capped by the tile count.
-static int configure(const void* kernel, const SmemPlan& sp, int64_t tiles, LaunchCfg* cfg) {
+// tmem_cols: TMEM columns a CTA of this launch allocates (the tcgen05 engine: kTcTmemCols; the step and VJP kernels
+// with the activation stash: stash_tmem_cols), 0 for kernels without tcgen05.alloc.
+static int configure(const void* kernel, const SmemPlan& sp, int64_t tiles, LaunchCfg* cfg, int tmem_cols = 0) {
   DeviceInfo di;
   if (int rc = device_info(&di)) return rc;
   size_t smem = (size_t)sp.floats * sizeof(float);
@@ -208,10 +210,11 @@ static int configure(const void* kernel, const SmemPlan& sp, int64_t tiles, Laun
   int occ = 0;
   e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, kTile, smem);
   if (e != cudaSuccess) return cuda_fail(e, "cudaOccupancyMaxActiveBlocksPerMultiprocessor");
-  if (sp.off_wmma >= 0) {
+  if (sp.off_wmma >= 0) tmem_cols = kTcTmemCols;
+  if (tmem_cols > 0) {
     // The occupancy query answers 1 for any kernel that contains tcgen05.alloc (it cannot know how
-    // many of the 512 TMEM columns a CTA takes; ours takes 32).  Size the persistent grid from the
-    // real limits instead: shared memory and registers.
+    // many of the 512 TMEM columns a CTA takes).  Size the persistent grid from the real limits
+    // instead: shared memory, registers and TMEM columns.
     cudaFuncAttributes fa;
     e = cudaFuncGetAttributes(&fa, kernel);
     if (e != cudaSuccess) return cuda_fail(e, "cudaFuncGetAttributes");
@@ -220,7 +223,7 @@ static int configure(const void* kernel, const SmemPlan& sp, int64_t tiles, Laun
     cudaDeviceGetAttribute(&regs_sm, cudaDevAttrMaxRegistersPerMultiprocessor, di.device);
     int by_smem = (int)(smem_sm / (smem + fa.sharedSizeBytes + 1024));
     int by_regs = regs_sm / (fa.numRegs * kTile > 0 ? fa.numRegs * kTile : 1);
-    int by_tmem = 512 / 32;
+    int by_tmem = 512 / tmem_cols;
     occ = by_smem < by_regs ? by_smem : by_regs;
     if (occ > by_tmem) occ = by_tmem;
   }
@@ -257,21 +260,22 @@ static int64_t partial_bytes(const FlowLayout& lay) {
   int64_t grad = ((int64_t)kMaxGrid * lay.total * sizeof(float) + 255) / 256 * 256;
   return kCounterBytes + loss + grad + frag_bytes(lay);
 }
-// Activation stash of the step kernel (warp-level engines, small flows): per CTA, per conditioner, 4 M float4 of hidden
-// activations + ceil((2 K + 10) / 4) float4 of located-spline state per thread (DeviceCtxMma::kStashChunks).  Sized for the largest persistent grid; it is re-written tile after tile and lives in L2.
-static int64_t stash_cta_floats(const FlowLayout& lay) {
-  if (!tc_available(lay)) return 0;
-  const int64_t per_cta = (int64_t)lay.L * (lay.D - 1) * (4 * lay.M + (2 * lay.K + 10 + 3) / 4) * kTile * 4;
-  if (per_cta * (int64_t)sizeof(float) > 64 * 1024) return 0;   // larger flows: recompute (the buffer would not stay in L2)
-  if (const char* e = getenv("CNFOT_STEP_STASH")) {             // tuning knob: 0 = always recompute
+// TMEM columns per CTA of the activation stash of the warp-MMA step and VJP kernels (warp_mlp.cuh: DeviceCtxMma): per
+// thread and conditioner, M tiles of 16 hidden activations + the located spline (2 K + 10 floats), rounded up to the
+// power of two tcgen05.alloc takes.  0 (recompute in the backward pass): other engines, flows over 128 columns (four
+// CTAs per SM share an SM's 512; such flows are also the only ones on the streamed plan), or CNFOT_STEP_STASH=0.
+// Non-zero selects the kernel instantiation with the stash (kEngMmaStash).
+static int stash_tmem_cols(const FlowLayout& lay, int engine) {
+  if (engine != kEngMma) return 0;
+  const int per_thread = lay.L * (lay.D - 1) * (16 * lay.M + 2 * lay.K + 10);
+  if (per_thread > 128) return 0;
+  if (const char* e = getenv("CNFOT_STEP_STASH")) {   // tuning knob: 0 = always recompute
     if (e[0] == '0') return 0;
   }
-  return per_cta;
+  int cols = 32;
+  while (cols < per_thread) cols <<= 1;
+  return cols;
 }
-constexpr int kStashMaxGrid = 6 * 148;   // the stash is sized for this many persistent CTAs (larger grids recompute)
-static int64_t stash_bytes(const FlowLayout& lay) { return stash_cta_floats(lay) * (int64_t)sizeof(float) * kStashMaxGrid; }
-// workspace of the step: [partials ... fragments | activation stash]
-static int64_t step_bytes(const FlowLayout& lay) { return partial_bytes(lay) + stash_bytes(lay); }
 static float* carve_frags(void* ws, const FlowLayout& lay) {
   return (float*)((char*)ws + partial_bytes(lay) - frag_bytes(lay));
 }
@@ -621,7 +625,7 @@ int64_t cnfot_flow_vjp_workspace_bytes(const cnfot_flow_desc* flow, int64_t rows
   FlowLayout lay;
   if (check_flow(flow, &lay)) return -1;
   if (use_wide(flow, lay)) return wide_flow_workspace_bytes(lay, rows, true);
-  return step_bytes(lay);   // partial results + the activation stash (seam 1 differentiates the rows it just evaluated)
+  return partial_bytes(lay);
 }
 
 static int flow_vjp_call(int dir, void* stream, const cnfot_flow_desc* flow, const float* weights,
@@ -661,9 +665,10 @@ static int flow_vjp_call(int dir, void* stream, const cnfot_flow_desc* flow, con
   SmemPlan sp;
   int engine;
   if (int rc = make_plan(lay, true, &sp, &engine)) return rc;
-  const void* kernel = find_flow_vjp_kernel(lay, engine);
+  const int stash_cols = stash_tmem_cols(lay, engine);   // seam 1 differentiates the rows it just evaluated
+  const void* kernel = find_flow_vjp_kernel(lay, engine, stash_cols > 0);
   LaunchCfg cfg;
-  if (int rc = configure(kernel, sp, (rows + kTile - 1) / kTile, &cfg)) return rc;
+  if (int rc = configure(kernel, sp, (rows + kTile - 1) / kTile, &cfg, stash_cols)) return rc;
   unsigned long long* counter;
   VjpArgs a;
   a.W = weights; a.frags = nullptr; a.in = in; a.cond = cond; a.cond_stride = cond_stride; a.rows = rows;
@@ -675,11 +680,7 @@ static int flow_vjp_call(int dir, void* stream, const cnfot_flow_desc* flow, con
   a.g_out = g_out; a.g_logdet = g_logdet; a.g_in = g_in; a.dir = dir; a.add_base = add_base;
   a.D = lay.D; a.L = lay.L; a.plan = sp;
   a.pb = carve_partials(workspace, &counter);
-  a.stash = nullptr;
-  a.stash_cta_floats = (engine == kEngMma || engine == kEngMmaStream) && cfg.grid <= kStashMaxGrid &&
-                               workspace_bytes >= step_bytes(lay)
-                           ? stash_cta_floats(lay) : 0;
-  if (a.stash_cta_floats > 0) a.stash = (float*)((char*)workspace + partial_bytes(lay));
+  a.stash_cols = stash_cols;
   void* args[] = {&a};
   cudaError_t e = cudaLaunchKernel(kernel, dim3(cfg.grid), dim3(kTile), args, cfg.smem, s);
   if (e != cudaSuccess) return cuda_fail(e, "flow_vjp_kernel launch");
@@ -747,7 +748,7 @@ static cudaError_t launch_step_kernel(const void* kernel, int grid, void** args,
 
 // ---- seam 3 ---------------------------------------------------------------------------
 static int64_t step_ws_bytes(const cnfot_flow_desc* flow, const FlowLayout& lay, int64_t rows_B, int64_t rows_b) {
-  return use_wide(flow, lay) ? wide_step_workspace_bytes(lay, rows_B, rows_b) : step_bytes(lay);
+  return use_wide(flow, lay) ? wide_step_workspace_bytes(lay, rows_B, rows_b) : partial_bytes(lay);
 }
 
 int64_t cnfot_mfc_step_workspace_bytes(const cnfot_flow_desc* flow, int64_t rows_B, int64_t rows_b,
@@ -869,8 +870,8 @@ static int mfc_step_impl(void* stream, const cnfot_flow_desc* flow, const cnfot_
   if (!weights || !workspace) return fail(CNFOT_ERR_ARG, "NULL buffer");
   if (!io.out && !io.stateful) return fail(CNFOT_ERR_ARG, "out is NULL");
   if (!io.rng && !io.t_batch_host) return fail(CNFOT_ERR_ARG, "t_batch is NULL");
-  if (workspace_bytes < step_bytes(lay)) return fail(CNFOT_ERR_WORKSPACE, "workspace too small: %lld < %lld",
-                                                     (long long)workspace_bytes, (long long)step_bytes(lay));
+  if (workspace_bytes < partial_bytes(lay)) return fail(CNFOT_ERR_WORKSPACE, "workspace too small: %lld < %lld",
+                                                        (long long)workspace_bytes, (long long)partial_bytes(lay));
   const char* err = nullptr;
   if (make_step_consts<float>(*problem, lay.D, (double)lambda, global_B, global_b, n_t, &a.pc, &err))
     return fail(CNFOT_ERR_ARG, "%s", err);
@@ -930,7 +931,8 @@ static int mfc_step_impl(void* stream, const cnfot_flow_desc* flow, const cnfot_
     latency = fit_tiles + (int64_t)n_t * ((rows_b + unit - 1) / unit) < 8 * 4 * 148;
     if (const char* e = getenv("CNFOT_STEP_LATENCY")) latency = e[0] != '0';
   }
-  const void* kernel = find_mfc_step_kernel(lay, engine, group > 1, latency);
+  const int stash_cols = stash_tmem_cols(lay, engine);
+  const void* kernel = find_mfc_step_kernel(lay, engine, group > 1, latency, stash_cols > 0);
   for (int i = 0; i < n_t; ++i)
     add(group > 1 ? kSegKineticSplit : kSegKinetic, kSlotKinetic, 0, 0, io.rng ? 0.f : io.t_batch_host[i], io.rng ? i : -1,
         io.latent_sub, kRowsNormal, io.row0_b, rows_b, group);
@@ -951,7 +953,7 @@ static int mfc_step_impl(void* stream, const cnfot_flow_desc* flow, const cnfot_
   a.salt_b = philox_salt(kDrawNormal, (uint64_t)global_b);
   a.salt_t = philox_salt(kDrawUniform, (uint64_t)n_t);
   LaunchCfg cfg;
-  if (int rc = configure(kernel, sp, (tiles * unit + kTile - 1) / kTile, &cfg)) return rc;
+  if (int rc = configure(kernel, sp, (tiles * unit + kTile - 1) / kTile, &cfg, stash_cols)) return rc;
   a.W = weights;
   a.frags = nullptr;
   if (engine == kEngMmaStream) {
@@ -960,9 +962,7 @@ static int mfc_step_impl(void* stream, const cnfot_flow_desc* flow, const cnfot_
     a.frags = fr;
   }
   a.D = lay.D; a.L = lay.L; a.plan = sp;
-  a.stash = nullptr;
-  a.stash_cta_floats = (engine == kEngMma || engine == kEngMmaStream) && cfg.grid <= kStashMaxGrid ? stash_cta_floats(lay) : 0;
-  if (a.stash_cta_floats > 0) a.stash = (float*)((char*)workspace + partial_bytes(lay));
+  a.stash_cols = stash_cols;
   // workspace / train state: [header: sync words, state words, loss row | partial gradient rows]
   TailArgs& t = a.tail;
   char* wsb = (char*)workspace;
@@ -1042,8 +1042,8 @@ int cnfot_workspace_register(void* stream, const cnfot_flow_desc* flow, void* wo
   if (int rc = check_flow(flow, &lay)) return rc;
   if (use_wide(flow, lay)) return fail(CNFOT_ERR_ARG, "persistent workspaces serve the fused per-row step kernel, not the wide-conditioner engine");
   if (!workspace) return fail(CNFOT_ERR_ARG, "NULL buffer");
-  if (workspace_bytes < step_bytes(lay)) return fail(CNFOT_ERR_WORKSPACE, "workspace too small: %lld < %lld",
-                                                     (long long)workspace_bytes, (long long)step_bytes(lay));
+  if (workspace_bytes < partial_bytes(lay)) return fail(CNFOT_ERR_WORKSPACE, "workspace too small: %lld < %lld",
+                                                        (long long)workspace_bytes, (long long)partial_bytes(lay));
   cudaError_t e = cudaMemsetAsync(workspace, 0, (size_t)kCounterBytes + (size_t)kStepRows * lay.total * sizeof(float),
                                   (cudaStream_t)stream);
   if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync");
@@ -1116,7 +1116,7 @@ int64_t cnfot_train_state_bytes(const cnfot_flow_desc* flow) {
   FlowLayout lay;
   if (check_flow(flow, &lay)) return -1;
   if (use_wide(flow, lay)) { fail(CNFOT_ERR_ARG, "no device-resident update for the wide-conditioner engine"); return -1; }
-  return step_bytes(lay);
+  return partial_bytes(lay);
 }
 
 int cnfot_train_state_init(void* stream, const cnfot_flow_desc* flow, void* state, int64_t state_bytes, uint64_t key,
@@ -1301,7 +1301,7 @@ int64_t cnfot_mfc_step_rng_host_workspace_bytes(const cnfot_flow_desc* flow) {
   FlowLayout lay;
   if (check_flow(flow, &lay)) return -1;
   if (use_wide(flow, lay)) { fail(CNFOT_ERR_ARG, "on-chip draws are not available on the wide-conditioner engine"); return -1; }
-  return align256(step_bytes(lay)) + align256((int64_t)lay.total * sizeof(float)) +
+  return align256(partial_bytes(lay)) + align256((int64_t)lay.total * sizeof(float)) +
          align256((int64_t)(lay.total + CNFOT_NUM_LOSS_SLOTS) * sizeof(float));
 }
 
@@ -1318,7 +1318,7 @@ int cnfot_mfc_step_rng_host(void* stream, const cnfot_flow_desc* flow, const cnf
                                           (long long)workspace_bytes, (long long)need);
   cudaStream_t s = (cudaStream_t)stream;
   char* p = (char*)workspace;
-  const int64_t ws_bytes = align256(step_bytes(lay));
+  const int64_t ws_bytes = align256(partial_bytes(lay));
   void* ws = p; p += ws_bytes;
   float* dW = (float*)p; p += align256((int64_t)lay.total * sizeof(float));
   float* dOut = (float*)p;

@@ -195,7 +195,8 @@ struct DeviceCtx {
   static constexpr bool kAccInGlobal = false;
   __device__ __forceinline__ void bind_partials(float*, bool = true) {}
   __device__ __forceinline__ void bind_frags(const float*) {}
-  __device__ __forceinline__ void bind_stash(float*) {}
+  __device__ __forceinline__ void stash_acquire(int, int, uint32_t*) {}
+  __device__ __forceinline__ void stash_release() {}
   __device__ __forceinline__ bool stash_on() const { return false; }   // the warp-level engines keep an activation stash
   static constexpr int H = Net::kH, M = Net::kM, Pp = Net::kPp;
   float* smem;

@@ -13,9 +13,11 @@ namespace cnfot {
 // shared memory (warp_mlp.cuh), 3 warp-level MMA streaming them from global memory; engines 1-3 exist
 // for hidden == 16 and num_bins == 5 only (tc_available()).
 const void* find_flow_eval_kernel(const FlowLayout& f, int engine = 0);
-const void* find_flow_vjp_kernel(const FlowLayout& f, int engine = 0);
+// stash (engine 2 only): the instantiation that keeps the activation stash in tensor memory (warp_mlp.cuh)
+const void* find_flow_vjp_kernel(const FlowLayout& f, int engine = 0, bool stash = false);
 // split: flow_kernels.cuh SPLIT; latency: the two-CTAs-per-SM instantiation of the streamed plan (LAT)
-const void* find_mfc_step_kernel(const FlowLayout& f, int engine = 0, bool split = false, bool latency = false);
+const void* find_mfc_step_kernel(const FlowLayout& f, int engine = 0, bool split = false, bool latency = false,
+                                 bool stash = false);
 const void* find_energy_kernel(const FlowLayout& f, int engine = 0);
 const void* find_density_kernel(const FlowLayout& f, int engine = 0);
 inline bool tc_available(const FlowLayout& f) { return f.H == 16 && f.K == 5 && f.D >= 2 && f.M <= 3; }

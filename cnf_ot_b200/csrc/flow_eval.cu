@@ -36,9 +36,15 @@ const void* find_flow_eval_kernel(const FlowLayout& f, int engine) {
   return nullptr;
 }
 
-const void* find_flow_vjp_kernel(const FlowLayout& f, int engine) {
+const void* find_flow_vjp_kernel(const FlowLayout& f, int engine, bool stash) {
   if (engine == kEngTc && tc_available(f)) {
     VJP_ENG_CASE(1, kEngTc) VJP_ENG_CASE(2, kEngTc) VJP_ENG_CASE(3, kEngTc)
+    return nullptr;
+  }
+  if (engine == kEngMma && tc_available(f) && stash) {
+    if (f.M == 2 && f.D == 2 && f.L == 2)
+      return (const void*)&flow_vjp_kernel<NetCfg<16, 5, 2>, Dims<2, 2>, kEngMmaStash>;
+    VJP_ENG_CASE(1, kEngMmaStash) VJP_ENG_CASE(2, kEngMmaStash) VJP_ENG_CASE(3, kEngMmaStash)
     return nullptr;
   }
   if (engine == kEngMma && tc_available(f)) {

@@ -14,8 +14,10 @@
 namespace cnfot {
 
 // CTA context by engine: 0 CUDA-core dense layers, 1 the tcgen05 engine (tc_engine.cuh),
-// 2 the warp-level tensor-core engine (warp_mlp.cuh); 1 and 2 exist for 16-wide networks
-enum Engine { kEngCuda = 0, kEngTc = 1, kEngMma = 2, kEngMmaStream = 3, kEngWide = 4 };
+// 2 the warp-level tensor-core engine (warp_mlp.cuh); 1 and 2 exist for 16-wide networks.
+// kEngMmaStash: the warp-level engine with the activation stash in tensor memory -- a kernel instantiation of its own
+// (step and VJP kernels only), so that no other kernel contains tcgen05 instructions.
+enum Engine { kEngCuda = 0, kEngTc = 1, kEngMma = 2, kEngMmaStream = 3, kEngWide = 4, kEngMmaStash = 5 };
 #ifndef CNFOT_MMA_MIN_CTAS
 #define CNFOT_MMA_MIN_CTAS 4
 #endif
@@ -43,6 +45,8 @@ template <class Net, int DC, int LC>
 struct CtxSelect<Net, kEngMma, DC, LC> { using type = DeviceCtxMma<Net, true, DC, LC>; };
 template <class Net, int DC, int LC>
 struct CtxSelect<Net, kEngMmaStream, DC, LC> { using type = DeviceCtxMma<Net, false>; };
+template <class Net, int DC, int LC>
+struct CtxSelect<Net, kEngMmaStash, DC, LC> { using type = DeviceCtxMma<Net, true, DC, LC, true>; };
 
 template <class Ctx>
 __device__ __forceinline__ void ctx_setup(Ctx& ctx, int D, int L, uint64_t* mbar, uint32_t* slot) {
@@ -138,8 +142,7 @@ struct VjpArgs {
   int D, L;
   SmemPlan plan;
   PartialBuf pb;
-  float* stash;                 // activation stash (warp-level engines; stash_cta_floats per CTA), or nullptr
-  long long stash_cta_floats;
+  int stash_cols;               // TMEM columns of the activation stash per CTA (warp-level engines), or 0
 };
 
 template <class Net, class DimsT, int ENG>
@@ -154,7 +157,7 @@ __global__ void __launch_bounds__(kTile, ENG >= kEngMma ? kMmaMinCtas : 1) flow_
   ctx.smem = smem; ctx.gW = a.W; ctx.p = a.plan;
   ctx.bind_partials(a.pb.grad + (int64_t)blockIdx.x * a.plan.total);
   ctx.bind_frags(a.frags);
-  ctx.bind_stash(a.stash ? a.stash + (size_t)blockIdx.x * a.stash_cta_floats : nullptr);
+  ctx.stash_acquire(a.stash_cols, a.L * (a.D - 1), &tc_slot);
   ctx_setup(ctx, a.D, a.L, &tc_mbar, &tc_slot);
   const RowTiles<float, Net> tl = make_row_tiles<Net>(smem, a.plan);
   const DimsT dm{a.D, a.L};
@@ -188,6 +191,7 @@ __global__ void __launch_bounds__(kTile, ENG >= kEngMma ? kMmaMinCtas : 1) flow_
     if (live && a.g_in)
       for (int i = 0; i < D; ++i) a.g_in[r * D + i] = g[i];
   }
+  ctx.stash_release();
   {
     float graw[Net::kPp];
 #pragma unroll
@@ -437,8 +441,7 @@ struct StepArgs {
   StepConsts<float> pc;
   int n_seg;
   int64_t n_tiles;     // 128-row tiles
-  float* stash;                 // activation stash of the warp-level engines (stash_cta_floats per CTA), or nullptr
-  long long stash_cta_floats;
+  int stash_cols;      // TMEM columns of the activation stash per CTA (warp-level engines), or 0
   unsigned long long key;       // on-chip draws (philox.cuh): key and step, or read from the train state
   unsigned long long salt_B, salt_Bc, salt_b, salt_t;   // key modifiers: normal (B, D), categorical (B,), normal (b, D), uniform (n_t,)
   uint32_t step;
@@ -674,7 +677,7 @@ mfc_step_kernel(const __grid_constant__ StepArgs a) {
   ctx.smem = smem; ctx.gW = a.W; ctx.p = a.plan;
   ctx.bind_partials(my_row, false);   // shared, pre-zeroed partial rows: the context must not clear them
   ctx.bind_frags(a.frags);
-  ctx.bind_stash(a.stash ? a.stash + (size_t)blockIdx.x * a.stash_cta_floats : nullptr);
+  ctx.stash_acquire(a.stash_cols, DimsT{a.D, a.L}.L() * (DimsT{a.D, a.L}.D() - 1), &tc_slot);
   ctx_setup(ctx, DimsT{a.D, a.L}.D(), DimsT{a.D, a.L}.L(), &tc_mbar, &tc_slot);   // compile-time shape where the kernel has one
   if (a.timeline && threadIdx.x == 0) { const unsigned long long now = global_timer_ns(); atomicMax(a.timeline + 1, now); atomicMax(a.timeline + 6, now - t_start); }   // last CTA is set up; longest setup
   const RowTiles<float, Net> tl = make_row_tiles<Net>(smem, a.plan);
@@ -748,7 +751,9 @@ mfc_step_kernel(const __grid_constant__ StepArgs a) {
     }
   }
   // Out of tiles: the next kernel of the stream may take the SM slots this grid frees from here on (every CTA of this
-  // grid is resident or done by the time the last one gets here, so the newcomers cannot keep any of them out).
+  // grid is resident or done by the time the last one gets here, so the newcomers cannot keep any of them out).  The
+  // stash's TMEM columns are freed first, so a newcomer never finds them held.
+  ctx.stash_release();
   asm volatile("griddepcontrol.launch_dependents;");
   if (a.timeline && threadIdx.x == 0) {   // this CTA ran out of tiles
     const unsigned long long now = global_timer_ns();

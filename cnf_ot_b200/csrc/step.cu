@@ -6,18 +6,19 @@
 namespace cnfot {
 
 const void* find_mfc_step_kernel_tc(const FlowLayout& f);
-const void* find_mfc_step_kernel_mma(const FlowLayout& f);
+const void* find_mfc_step_kernel_mma(const FlowLayout& f, bool stash);
 const void* find_mfc_step_kernel_mma_stream(const FlowLayout& f);
 const void* find_mfc_step_kernel_cuda(const FlowLayout& f);
 const void* find_mfc_step_kernel_tc_split(const FlowLayout& f);
-const void* find_mfc_step_kernel_mma_split(const FlowLayout& f);
+const void* find_mfc_step_kernel_mma_split(const FlowLayout& f, bool stash);
 const void* find_mfc_step_kernel_mma_stream_split(const FlowLayout& f);
 const void* find_mfc_step_kernel_mma_stream_lat(const FlowLayout& f);
 const void* find_mfc_step_kernel_cuda_split(const FlowLayout& f);
 
-const void* find_mfc_step_kernel(const FlowLayout& f, int engine, bool split, bool latency) {
+const void* find_mfc_step_kernel(const FlowLayout& f, int engine, bool split, bool latency, bool stash) {
   if (engine == kEngTc && tc_available(f)) return split ? find_mfc_step_kernel_tc_split(f) : find_mfc_step_kernel_tc(f);
-  if (engine == kEngMma && tc_available(f)) return split ? find_mfc_step_kernel_mma_split(f) : find_mfc_step_kernel_mma(f);
+  if (engine == kEngMma && tc_available(f))
+    return split ? find_mfc_step_kernel_mma_split(f, stash) : find_mfc_step_kernel_mma(f, stash);
   if (engine == kEngMmaStream && tc_available(f))
     return split ? find_mfc_step_kernel_mma_stream_split(f)
                  : (latency ? find_mfc_step_kernel_mma_stream_lat(f) : find_mfc_step_kernel_mma_stream(f));

@@ -242,7 +242,8 @@ __device__ __forceinline__ float* dyn_smem_ptr() {
 // plan is a compile-time constant, so the tile / weight / fragment / knot addresses the engine needs all the time are
 // immediates (+ the warp index) instead of members of a context that lives in the caller's local memory and has to be
 // re-loaded after every asm memory clobber (a quarter of the kernel's long-scoreboard stalls, tools/ncu_stall_lines.py).
-template <class Net, bool RES, int DC = 0, int LC = 0>
+// STASH: the kernel keeps the activation stash (below) in tensor memory; false: no tcgen05 instruction is compiled in.
+template <class Net, bool RES, int DC = 0, int LC = 0, bool STASH = false>
 struct DeviceCtxMma {
   using NetT = Net;
   using Ref = WRef<RES>;
@@ -277,43 +278,106 @@ struct DeviceCtxMma {
   const float* gfrag;   // streamed plan: the fragment buffer in global memory
   Ref w_ref, frag_ref;  // blob and fragments (shared-window address or global pointer)
   uint32_t s_wt;        // shared-window address of this warp's tiles
-  // Activation stash (this CTA's slice of a global buffer that stays in L2): the forward pass of a row that is
-  // differentiated right away (KL / reverse-KL / potential rows: 97 % of a step) leaves every conditioner's hidden
-  // activations (as the warp holds them: MMA fragments) and the located spline (SplineState of the thread's row: softmax
-  // probabilities, the gathered knots, slope logits) here, and the backward pass reads them back instead of evaluating
-  // the conditioner and normalising the knots a second time.  nullptr: recompute.
-  float* stash = nullptr;
+  // Activation stash in tensor memory: the forward pass of a row that is differentiated right away (KL / reverse-KL /
+  // potential rows: 97 % of a step) leaves every conditioner's hidden activations (as the warp holds them: MMA
+  // fragments) and the located spline (SplineState of the thread's row: softmax probabilities, the gathered knots, slope
+  // logits) here, and the backward pass reads them back instead of evaluating the conditioner and normalising the knots
+  // a second time.  The stash is strictly per thread, which is the tcgen05.ld / tcgen05.st 32x32b shape: thread i of
+  // warp w owns TMEM lane 32 w + i.  Columns of a thread (nc = L (D - 1) conditioners, c = layer (D - 1) + d - 1; every
+  // 16-column access starts on a 16-column boundary):
+  //   [16 (c M + m), +16)          hidden activations m of conditioner c (A order)
+  //   [16 (nc M + c), +16)         located spline of conditioner c, floats 0..15
+  //   [16 nc (M + 1) + 4 c, +4)    its floats 16..19
+  // stash_nc == 0: no stash, the backward pass recomputes.
   static constexpr int kStateFloats = 2 * Net::kK + 10;
-  static constexpr int kStateChunks = (kStateFloats + 3) / 4;
-  static constexpr int kStashChunks = 4 * M + kStateChunks;   // float4 per thread and conditioner
-  static constexpr int kStashCondFloats = kStashChunks * kTile * 4;
-  __device__ __forceinline__ void bind_stash(float* q) { stash = q; }
-  __device__ __forceinline__ bool stash_on() const { return stash != nullptr; }
-  __device__ __forceinline__ float* stash_of(int D, int layer, int d) const {
-    return stash + (size_t)(layer * (D - 1) + d - 1) * kStashCondFloats + threadIdx.x * 4;
+  static_assert(kStateFloats == 20, "the stash layout holds a located spline of 5 bins");
+  uint32_t stash_t = 0;   // TMEM address of lane 32 w, column 0 (w: the calling thread's warp)
+  int stash_nc = 0;
+  int stash_cols = 0;     // columns allocated by this CTA
+  __device__ __forceinline__ bool stash_on() const { return STASH && stash_nc != 0; }
+  __device__ __forceinline__ int stash_ncond() const {
+    if constexpr (kConstPlan) return LC * (DC - 1);
+    else return stash_nc;
   }
-  __device__ __forceinline__ static void stash_put(float* q, int chunk0, const float (&v)[2][2][4]) {
-#pragma unroll
-    for (int c = 0; c < 4; ++c)
-      __stcg(reinterpret_cast<float4*>(q + (chunk0 + c) * kTile * 4),
-             make_float4(v[c >> 1][c & 1][0], v[c >> 1][c & 1][1], v[c >> 1][c & 1][2], v[c >> 1][c & 1][3]));
+  __device__ __forceinline__ static int stash_cond(int D, int layer, int d) { return layer * (D - 1) + d - 1; }
+  // cols: a power of two >= 32 (the host launches a STASH kernel only with the stash on).  One warp allocates, every
+  // thread leaves with the address.  A CTA allocates once, so it gives up its allocation permit right away.
+  __device__ __forceinline__ void stash_acquire(int cols, int n_cond, uint32_t* slot) {
+    if constexpr (STASH) {
+      if (threadIdx.x < 32) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
+                     ::"r"((uint32_t)__cvta_generic_to_shared(slot)), "r"(cols) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+      }
+      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+      __syncthreads();
+      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      stash_t = *slot + ((threadIdx.x & ~31u) << 16);
+      stash_nc = n_cond;
+      stash_cols = cols;
+    }
   }
+  // Every thread of the CTA calls this once it has no rows left: the columns go back to the SM at once (a kernel that
+  // is launched behind this one may then allocate them while this CTA is still in its epilogue).
+  __device__ __forceinline__ void stash_release() {
+    if constexpr (STASH) {
+      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+      __syncthreads();
+      if (threadIdx.x < 32) {
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(stash_t), "r"(stash_cols) : "memory");
+      }
+      stash_nc = 0;
+      stash_cols = 0;
+    }
+  }
+  __device__ __forceinline__ static void tmem_st16(uint32_t ta, const float* v) {
+    asm volatile(
+        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};"
+        ::"r"(ta), "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7]), "f"(v[8]),
+          "f"(v[9]), "f"(v[10]), "f"(v[11]), "f"(v[12]), "f"(v[13]), "f"(v[14]), "f"(v[15])
+        : "memory");
+  }
+  __device__ __forceinline__ static void tmem_st4(uint32_t ta, const float* v) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};"
+                 ::"r"(ta), "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3]) : "memory");
+  }
+  // load and wait in one statement: the outputs cannot be used before tcgen05.wait::ld has returned
+  __device__ __forceinline__ static void tmem_ld16(uint32_t ta, float* v) {
+    asm volatile(
+        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];\n\t"
+        "tcgen05.wait::ld.sync.aligned;"
+        : "=f"(v[0]), "=f"(v[1]), "=f"(v[2]), "=f"(v[3]), "=f"(v[4]), "=f"(v[5]), "=f"(v[6]), "=f"(v[7]), "=f"(v[8]),
+          "=f"(v[9]), "=f"(v[10]), "=f"(v[11]), "=f"(v[12]), "=f"(v[13]), "=f"(v[14]), "=f"(v[15])
+        : "r"(ta) : "memory");
+  }
+  __device__ __forceinline__ static void tmem_ld16_4(uint32_t ta16, uint32_t ta4, float* v) {
+    asm volatile(
+        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%20];\n\t"
+        "tcgen05.ld.sync.aligned.32x32b.x4.b32 {%16,%17,%18,%19}, [%21];\n\t"
+        "tcgen05.wait::ld.sync.aligned;"
+        : "=f"(v[0]), "=f"(v[1]), "=f"(v[2]), "=f"(v[3]), "=f"(v[4]), "=f"(v[5]), "=f"(v[6]), "=f"(v[7]), "=f"(v[8]),
+          "=f"(v[9]), "=f"(v[10]), "=f"(v[11]), "=f"(v[12]), "=f"(v[13]), "=f"(v[14]), "=f"(v[15]), "=f"(v[16]),
+          "=f"(v[17]), "=f"(v[18]), "=f"(v[19])
+        : "r"(ta16), "r"(ta4) : "memory");
+  }
+  __device__ __forceinline__ uint32_t stash_hidden(int c, int m) const { return stash_t + 16 * (c * M + m); }
   // the located spline of the calling thread's row (after rqs_locate_raw in the forward pass)
   __device__ __forceinline__ void stash_state(int D, int layer, int d, const SplineState<float, Net::kK>& st) const {
-    constexpr int K = Net::kK;
-    float b[kStateChunks * 4];
-#pragma unroll
-    for (int k = 0; k < K; ++k) { b[k] = st.pw[k]; b[K + k] = st.ph[k]; }
-    b[2 * K] = st.x0; b[2 * K + 1] = st.x1; b[2 * K + 2] = st.y0; b[2 * K + 3] = st.y1;
-    b[2 * K + 4] = st.d0; b[2 * K + 5] = st.d1; b[2 * K + 6] = st.u0; b[2 * K + 7] = st.u1;
-    b[2 * K + 8] = st.u_tail;
-    b[2 * K + 9] = __int_as_float(st.idx | (st.tail << 8));
-#pragma unroll
-    for (int j = kStateFloats; j < kStateChunks * 4; ++j) b[j] = 0.f;
-    float* q = stash_of(D, layer, d) + 4 * M * kTile * 4;
-#pragma unroll
-    for (int c = 0; c < kStateChunks; ++c)
-      __stcg(reinterpret_cast<float4*>(q + c * kTile * 4), make_float4(b[4 * c], b[4 * c + 1], b[4 * c + 2], b[4 * c + 3]));
+    if constexpr (STASH) {
+      constexpr int K = Net::kK;
+      float b[kStateFloats];
+  #pragma unroll
+      for (int k = 0; k < K; ++k) { b[k] = st.pw[k]; b[K + k] = st.ph[k]; }
+      b[2 * K] = st.x0; b[2 * K + 1] = st.x1; b[2 * K + 2] = st.y0; b[2 * K + 3] = st.y1;
+      b[2 * K + 4] = st.d0; b[2 * K + 5] = st.d1; b[2 * K + 6] = st.u0; b[2 * K + 7] = st.u1;
+      b[2 * K + 8] = st.u_tail;
+      b[2 * K + 9] = __int_as_float(st.idx | (st.tail << 8));
+      const int c = stash_cond(D, layer, d), nc = stash_ncond();
+      __syncwarp();   // the .aligned stores need the whole warp (the spline's search branches per row)
+      tmem_st16(stash_t + 16 * (nc * M + c), b);
+      tmem_st4(stash_t + 16 * nc * (M + 1) + 4 * c, b + 16);
+    }
   }
 
   bool clear_acc;       // setup() zeroes the partial row (false: rows shared between CTAs, cleared by the caller)
@@ -504,7 +568,7 @@ struct DeviceCtxMma {
   // put: also leave them in the activation stash for cond_restore (the caller adds the located spline: stash_state).
   __device__ __forceinline__ void cond_forward(int D, int layer, int d, float tval, const float* cvec,
                                                float* theta, bool keep, bool put = false) const {
-    float* sq = put ? stash_of(D, layer, d) : nullptr;
+    const int sc = stash_cond(D, layer, d);
     const MmaLane ln;
     const uint32_t wt = swt();
     const int n_in = d + 1, mlp = layer * (D - 1) + d - 1;
@@ -541,7 +605,7 @@ struct DeviceCtxMma {
       __syncwarp();   // the previous conditioner's readers are done with the tiles
       store_a(wt, ln, a);
     }
-    if (put) stash_put(sq, 0, a);
+    if (STASH && put) tmem_st16(stash_hidden(sc, 0), &a[0][0][0]);
     // bias of dense matrix m: compact copy = right after b0; blob = after its matrix
     Ref bm = RES ? b0 + H : b0 + (H + H * H);
 #pragma unroll
@@ -549,7 +613,7 @@ struct DeviceCtxMma {
       dense16(a, frag + (m - 1) * kFragFloats, bm, ln, x);
       relu_to_a(x, a);
       if (keep) store_a(wt + m * kWtFloats * 4, ln, a);
-      if (put) stash_put(sq, 4 * m, a);
+      if (STASH && put) tmem_st16(stash_hidden(sc, m), &a[0][0][0]);
       bm = bm + (RES ? H : H * H + H);
     }
     dense16(a, frag + (M - 1) * kFragFloats, bm, ln, x);
@@ -562,42 +626,36 @@ struct DeviceCtxMma {
 
   // What cond_forward(keep = true) + rqs_locate_raw leave behind -- hidden activations in the warp's tiles, the located
   // spline of the calling thread's row -- read back from the activation stash the forward pass of the same rows filled
-  // (cond_forward(put = true), stash_state).  Every load is issued before the first use: ONE L2 round trip.
+  // (cond_forward(put = true), stash_state).  One 16-column load per tile goes straight into the tile, so only 16 (20
+  // for the spline) of the values are in registers at a time.
   __device__ __forceinline__ void cond_restore(int D, int layer, int d, SplineState<float, Net::kK>& st, float min_slope) const {
-    constexpr int K = Net::kK;
-    const MmaLane ln;
-    const uint32_t wt = swt();
-    const float* sq = stash_of(D, layer, d);
-    float4 f[kStashChunks];
-#pragma unroll
-    for (int c = 0; c < kStashChunks; ++c) f[c] = __ldcg(reinterpret_cast<const float4*>(sq + c * kTile * 4));
-    __syncwarp();   // the previous conditioner's readers are done with the tiles
-#pragma unroll
-    for (int m = 0; m < M; ++m) {
-      float a[2][2][4];
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        const float4 v = f[4 * m + c];
-        a[c >> 1][c & 1][0] = v.x; a[c >> 1][c & 1][1] = v.y; a[c >> 1][c & 1][2] = v.z; a[c >> 1][c & 1][3] = v.w;
+    if constexpr (STASH) {
+      constexpr int K = Net::kK;
+      const MmaLane ln;
+      const uint32_t wt = swt();
+      const int c = stash_cond(D, layer, d), nc = stash_ncond();
+      __syncwarp();   // the previous conditioner's readers are done with the tiles; the warp is converged for .aligned
+      // the stores of the forward pass have completed (they were issued a whole pass ago: this does not wait)
+      asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+  #pragma unroll
+      for (int m = 0; m < M; ++m) {
+        float a[2][2][4];
+        tmem_ld16(stash_hidden(c, m), &a[0][0][0]);
+        store_a(wt + m * kWtFloats * 4, ln, a);
       }
-      store_a(wt + m * kWtFloats * 4, ln, a);
+      float b[kStateFloats];
+      tmem_ld16_4(stash_t + 16 * (nc * M + c), stash_t + 16 * nc * (M + 1) + 4 * c, b);
+  #pragma unroll
+      for (int k = 0; k < K; ++k) { st.pw[k] = b[k]; st.ph[k] = b[K + k]; }
+      st.x0 = b[2 * K]; st.x1 = b[2 * K + 1]; st.y0 = b[2 * K + 2]; st.y1 = b[2 * K + 3];
+      st.d0 = b[2 * K + 4]; st.d1 = b[2 * K + 5]; st.u0 = b[2 * K + 6]; st.u1 = b[2 * K + 7];
+      st.u_tail = b[2 * K + 8];
+      const int it = __float_as_int(b[2 * K + 9]);
+      st.idx = it & 0xff;
+      st.tail = it >> 8;
+      st.s_tail = st.d0;
+      if (st.tail == 2) st.s_tail = softplus(st.u_tail) + min_slope;
     }
-    float b[kStateChunks * 4];
-#pragma unroll
-    for (int c = 0; c < kStateChunks; ++c) {
-      const float4 v = f[4 * M + c];
-      b[4 * c] = v.x; b[4 * c + 1] = v.y; b[4 * c + 2] = v.z; b[4 * c + 3] = v.w;
-    }
-#pragma unroll
-    for (int k = 0; k < K; ++k) { st.pw[k] = b[k]; st.ph[k] = b[K + k]; }
-    st.x0 = b[2 * K]; st.x1 = b[2 * K + 1]; st.y0 = b[2 * K + 2]; st.y1 = b[2 * K + 3];
-    st.d0 = b[2 * K + 4]; st.d1 = b[2 * K + 5]; st.u0 = b[2 * K + 6]; st.u1 = b[2 * K + 7];
-    st.u_tail = b[2 * K + 8];
-    const int it = __float_as_int(b[2 * K + 9]);
-    st.idx = it & 0xff;
-    st.tail = it >> 8;
-    st.s_tail = st.d0;
-    if (st.tail == 2) st.s_tail = softplus(st.u_tail) + min_slope;
   }
 
   // 4 per-thread partial sums (columns 2t, 2t+1, 8+2t, 9+2t of a 16-wide row) -> summed over the

@@ -1,7 +1,9 @@
-"""profiles/traffic.json from ncu reports (run after every kernel change; bench.py refuses a file whose source hash
-differs from the sources the loaded library was built from):
+"""profiles/traffic.json from a counter capture of the step kernel (run after every kernel change; bench.py refuses a
+file whose source hash differs from the sources the loaded library was built from):
 
-  python tools/make_traffic.py <step.ncu-rep> [<dense_tc.ncu-rep>]
+  python tools/make_traffic.py <step.ncu-rep | capture.json> [<dense_tc.ncu-rep>]
+
+capture.json: written by tools/capture_counters.py (CUPTI range profiler); it must carry the hash of the sources here.
 
 Records, per launch of mfc_step_kernel (BASELINE cfg 2): dram__bytes_read.sum + dram__bytes_write.sum and
 smsp__inst_executed.sum, plus the hash of cnf_ot_b200/csrc the capture belongs to (bench.kernel_fingerprint)."""
@@ -36,18 +38,27 @@ def num(v, unit):
 
 def main():
   step_rep = sys.argv[1]
-  ks, units = raw(step_rep)
-  k = next(r for r in ks if "mfc_step_kernel" in r["Kernel Name"])
-  rd = num(k["dram__bytes_read.sum"], units["dram__bytes_read.sum"])
-  wr = num(k["dram__bytes_write.sum"], units["dram__bytes_write.sum"])
-  insts = num(k["smsp__inst_executed.sum"], units["smsp__inst_executed.sum"])
+  if step_rep.endswith(".json"):
+    cap = json.load(open(step_rep))
+    if cap["csrc_sha16"] != fingerprint():
+      sys.exit(f"{step_rep} was captured from other kernel sources ({cap['csrc_sha16']} != {fingerprint()})")
+    m = cap["metrics"]
+    rd, wr, insts = m["dram__bytes_read.sum"], m["dram__bytes_write.sum"], m["smsp__inst_executed.sum"]
+    how = f"{cap['tool']}, {cap['gpu']}"
+  else:
+    ks, units = raw(step_rep)
+    k = next(r for r in ks if "mfc_step_kernel" in r["Kernel Name"])
+    rd = num(k["dram__bytes_read.sum"], units["dram__bytes_read.sum"])
+    wr = num(k["dram__bytes_write.sum"], units["dram__bytes_write.sum"])
+    insts = num(k["smsp__inst_executed.sum"], units["smsp__inst_executed.sum"])
+    how = "ncu --set full --clock-control none"
   tpath = os.path.join(ROOT, "profiles", "traffic.json")
   old = json.load(open(tpath)) if os.path.exists(tpath) else {}
   tj = {
     "csrc_sha16": fingerprint(),
     "mfc_step_kernel_dram_bytes_per_launch": int(rd + wr),
     "mfc_step_kernel_warp_insts_per_launch": int(insts),
-    "source": f"{os.path.basename(step_rep)} (ncu --set full --clock-control none, one launch of the cfg-2 step: dram__bytes_read.sum "
+    "source": f"{os.path.basename(step_rep)} ({how}, one launch of the cfg-2 step: dram__bytes_read.sum "
               f"{int(rd)} + dram__bytes_write.sum {int(wr)}; smsp__inst_executed.sum); written by tools/make_traffic.py",
   }
   for key in ("dense_tc_kernel_256_1_dram_bytes_per_launch", "dense_tc_kernel_source"):
