@@ -1419,7 +1419,7 @@ int cnfot_kinetic_energy(void* stream, const cnfot_flow_desc* flow, const float*
 int64_t cnfot_density_workspace_bytes(const cnfot_flow_desc* flow, int32_t n_t) {
   FlowLayout lay;
   if (check_flow(flow, &lay)) return -1;
-  if (use_wide(flow, lay)) { fail(CNFOT_ERR_ARG, "density evaluation runs on the fused kernels only"); return -1; }
+  if (use_wide(flow, lay)) return wide_density_workspace_bytes(lay, n_t);
   return partial_bytes(lay) + ((int64_t)(n_t > 0 ? n_t : 0) * (int64_t)sizeof(float) + 255) / 256 * 256 + 256;
 }
 
@@ -1427,8 +1427,9 @@ static int density_call(void* stream, const cnfot_flow_desc* flow, const float* 
                         int32_t n_t, double* sq_err, void* workspace, int64_t workspace_bytes) {
   FlowLayout lay;
   if (int rc = check_flow(flow, &lay)) return rc;
-  if (use_wide(flow, lay)) return fail(CNFOT_ERR_ARG, "density evaluation runs on the fused kernels only");
-  if (int rc = check_fused(flow, lay)) return rc;
+  const bool wide = use_wide(flow, lay);
+  if (!wide)
+    if (int rc = check_fused(flow, lay)) return rc;
   if (!weights || !workspace) return fail(CNFOT_ERR_ARG, "NULL buffer");
   if (a.with_ref && (!sq_err || !(a.var0 > 0.f) || !(a.var1 > 0.f))) return fail(CNFOT_ERR_ARG, "reference density: need sq_err and positive variances");
   const int64_t need = cnfot_density_workspace_bytes(flow, n_t);
@@ -1436,6 +1437,17 @@ static int density_call(void* stream, const cnfot_flow_desc* flow, const float* 
   cudaStream_t s = (cudaStream_t)stream;
   if (a.n == 0) {
     if (sq_err) { cudaError_t e = cudaMemsetAsync(sq_err, 0, sizeof(double), s); if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync"); }
+    return 0;
+  }
+  if (wide) {
+    const char* what = "";
+    cudaError_t we = a.mode == 0
+        ? wide_density_grid(s, lay, spline_consts(flow), weights, t_host, n_t, a.x_min, a.x_step, a.y_min, a.y_step, a.nx,
+                            a.ny, a.density, a.with_ref, a.mix, a.var0, a.var1, sq_err, workspace, &what)
+        : wide_density_mc(s, lay, spline_consts(flow), weights, a.cond, a.key_n, a.step, a.n, a.samples, a.density,
+                          a.with_ref, a.mix, a.var0, a.var1, sq_err, workspace, &what);
+    if (we != cudaSuccess) return cuda_fail(we, what);
+    g_last_launch[0] = 0; g_last_launch[1] = 0; g_last_launch[2] = 0; g_last_launch[3] = kEngWide;
     return 0;
   }
   float* t_dev = (float*)((char*)workspace + partial_bytes(lay));

@@ -314,7 +314,6 @@ __global__ void __launch_bounds__(kTile, ENG >= kEngMma ? kMmaMinCtas : 1) densi
   double loss[kNumSlots];
 #pragma unroll
   for (int s = 0; s < kNumSlots; ++s) loss[s] = 0.0;
-  const float half_log_2pi = 0.91893853320467274178f;
   for (int64_t tile = blockIdx.x; tile * kTile < a.n; tile += gridDim.x) {   // uniform cost per point: static tiles
     const int64_t r = tile * kTile + ctx.row_in_tile();
     const bool live = r < a.n;   // every thread runs the pass: the contexts have CTA / warp barriers
@@ -345,11 +344,7 @@ __global__ void __launch_bounds__(kTile, ENG >= kEngMma ? kMmaMinCtas : 1) densi
     const float p = m_exp(lp);
     if (a.density) a.density[r] = p;
     if (a.with_ref) {
-      float r2 = 0.f;
-      for (int i = 0; i < D; ++i) r2 += y[i] * y[i];
-      const float p0 = m_exp(-0.5f * r2 / a.var0 - (float)D * (half_log_2pi + 0.5f * m_log(a.var0)));
-      const float p1 = m_exp(-0.5f * r2 / a.var1 - (float)D * (half_log_2pi + 0.5f * m_log(a.var1)));
-      const float e = p - (p0 * (1.f - a.mix) + p1 * a.mix);
+      const float e = ref_mixture_error(p, y, D, a.mix, a.var0, a.var1);
       loss[kSlotKinetic] += (double)e * (double)e;
     }
   }

@@ -424,4 +424,17 @@ CNFOT_HD T base_log_prob(const T* x, int D) {
   return (T)-0.5 * acc - (T)0.91893853320467274178 * (T)D;
 }
 
+// p - ((1 - mix) N(y; 0, var0 I) + mix N(y; 0, var1 I)): the error of a density p at y against the reference density of
+// the fp evaluation (solvers.py:238-252,270-276), for density_kernel (flow_kernels.cuh) and the wide engine's density head
+// (wide.cu)
+CNFOT_HD float ref_mixture_error(float p, const float* y, int D, float mix, float var0, float var1) {
+  const float half_log_2pi = 0.91893853320467274178f;
+  float r2 = 0.f;
+  for (int i = 0; i < D; ++i) r2 += y[i] * y[i];
+  const float p0 = m_exp(-0.5f * r2 / var0 - (float)D * (half_log_2pi + 0.5f * m_log(var0)));
+  const float p1 = m_exp(-0.5f * r2 / var1 - (float)D * (half_log_2pi + 0.5f * m_log(var1)));
+  // the contraction nvcc made of p0 * (1 - mix) + p1 * mix written inline in density_kernel: its code is unchanged
+  return p - fmaf(p1, mix, p0 * (1.f - mix));
+}
+
 }  // namespace cnfot

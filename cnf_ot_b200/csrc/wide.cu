@@ -27,6 +27,7 @@
 #include <stdlib.h>
 
 #include "dense_tc.h"
+#include "philox.cuh"
 #include "wide.h"
 
 namespace cnfot {
@@ -724,6 +725,62 @@ wide_sumsq_kernel(const float* __restrict__ V, int64_t count, double weight, dou
 }
 __global__ void wide_energy_out_kernel(const double* __restrict__ slots, double* __restrict__ out) {
   if (threadIdx.x == 0) out[0] = slots[kSlotKinetic];
+}
+
+// ---- densities on a grid / at Monte-Carlo samples (density_kernel of flow_kernels.cuh on a chunk) -----------------
+struct DensityPoints {
+  int mode;                          // 0 grid, 1 Monte-Carlo
+  int nx, ny;                        // grid: flat point r = (ti, iy, ix)
+  double x_min, x_step, y_min, y_step;
+  const float* t_dev;                // grid: (n_t) times
+  uint64_t key_n;                    // Monte-Carlo: Philox key of the (n, D) normal draw
+  uint32_t step;
+  float cond;                        // Monte-Carlo: the time
+};
+// points [r0, r0 + n) into the chunk: S[0] = [point | t | 0 ..], S[1..L] = [0 | t | 0 ..] (wide_init_kernel's layout);
+// a grid chunk may cross a time boundary, so t is per row
+__global__ void __launch_bounds__(kThreads)
+wide_density_init_kernel(DensityPoints dp, int64_t r0, int64_t n, int D, int Kx, int L, int64_t state_stride,
+                         float* __restrict__ S) {
+  const int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (r >= n) return;
+  const int64_t g = r0 + r;
+  float* s0 = S + r * Kx;
+  float t;
+  if (dp.mode == 0) {
+    const int64_t per_t = (int64_t)dp.nx * dp.ny;
+    const int ti = (int)(g / per_t);
+    const int64_t q = g - (int64_t)ti * per_t;
+    const int iy = (int)(q / dp.nx), ix = (int)(q - (int64_t)iy * dp.nx);
+    s0[0] = (float)(dp.x_min + (double)ix * dp.x_step);
+    s0[1] = (float)(dp.y_min + (double)iy * dp.y_step);
+    t = dp.t_dev[ti];
+  } else {
+    philox_row(dp.key_n, dp.key_n, dp.step, kRowsNormal, (uint64_t)g, D, s0);
+    t = dp.cond;
+  }
+  for (int s = 0; s <= L; ++s) {
+    float* row = S + (int64_t)s * state_stride + r * Kx;
+    for (int c = s == 0 ? D : 0; c < Kx; ++c) row[c] = c == D ? t : 0.f;
+  }
+}
+// lp = log N(Z) + ld_sign LD (grid: Z = latent output, +ildj; Monte-Carlo: Z = latent input, -fldj); density = exp(lp) and,
+// with_ref, the squared error at the points Y against the reference mixture, summed in double into `slot`
+__global__ void __launch_bounds__(kThreads)
+wide_density_head_kernel(const float* __restrict__ Z, const float* __restrict__ Y, const float* __restrict__ LD,
+                         float ld_sign, int64_t n, int D, int Kx, float* __restrict__ density, int with_ref, float mix,
+                         float var0, float var1, double* __restrict__ slot) {
+  const int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  double sq = 0.0;
+  if (r < n) {
+    const float p = m_exp(base_log_prob<float>(Z + r * Kx, D) + ld_sign * LD[r]);
+    if (density) density[r] = p;
+    if (with_ref) {
+      const float e = ref_mixture_error(p, Y + r * Kx, D, mix, var0, var1);
+      sq = (double)e * (double)e;
+    }
+  }
+  if (with_ref) block_add(sq, slot);
 }
 
 // ---- batched passes: several flow passes that start from the same rows share ONE chunk ---------------------------
@@ -1598,6 +1655,81 @@ cudaError_t wide_kinetic_energy(cudaStream_t s, const FlowLayout& lay, const Spl
   }
   if (what) *what = e.what;
   return e.err;
+}
+
+int64_t wide_density_workspace_bytes(const FlowLayout& lay, int n_t) {
+  return carve(nullptr, lay, chunk_rows(), false, 1, nullptr) + round_up64((int64_t)(n_t > 0 ? n_t : 0) * (int64_t)sizeof(float), 256);
+}
+
+namespace {
+
+// the chunk loop of both density modes: one flow pass per chunk (grid: log-prob direction from the points; Monte-Carlo:
+// sample direction from the latent draw), then the head
+cudaError_t run_density(cudaStream_t s, const FlowLayout& lay, const SplineConsts<float>& sc, const float* weights,
+                        const DensityPoints& dp, int64_t n, float* samples, float* density, int with_ref, float mix,
+                        float var0, float var1, double* sq_err, void* workspace, const char** what) {
+  WideEngine e;
+  e.s = s; e.sc = sc; e.W = weights; e.grad = nullptr;
+  carve(workspace, lay, chunk_rows(), false, 1, &e);
+  if (with_ref) e.check(cudaMemsetAsync(e.slots, 0, kNumSlots * sizeof(double), s), "cudaMemsetAsync");
+  launch_prep(e, false);
+  const int D = e.wd.D, Kx = e.wd.Kx, L = e.wd.L;
+  const int dir = dp.mode == 0 ? 1 : 0;
+  for (int64_t r0 = 0; r0 < n && e.ok(); r0 += e.R) {
+    const int64_t m = n - r0 < e.R ? n - r0 : e.R;
+    wide_density_init_kernel<<<WideEngine::blocks_for(m), kThreads, 0, s>>>(dp, r0, m, D, Kx, L, e.state_stride(), e.S[0]);
+    e.check_launch("wide_density_init_kernel launch");
+    e.flow_pass<5>(dir, 0, m);
+    if (!e.ok()) break;
+    if (samples) {
+      wide_extract_kernel<<<WideEngine::grid_for(m * D), kThreads, 0, s>>>(e.state(0, L), m, D, Kx, samples + r0 * D);
+      e.check_launch("wide_extract_kernel launch");
+    }
+    if (density || with_ref) {
+      const float* Z = dir == 1 ? e.state(0, L) : e.state(0, 0);
+      const float* Y = dir == 1 ? e.state(0, 0) : e.state(0, L);
+      wide_density_head_kernel<<<WideEngine::blocks_for(m), kThreads, 0, s>>>(
+          Z, Y, e.LD[0], dir == 1 ? 1.f : -1.f, m, D, Kx, density ? density + r0 : nullptr, with_ref, mix, var0, var1,
+          e.slots + kSlotKinetic);
+      e.check_launch("wide_density_head_kernel launch");
+    }
+  }
+  if (with_ref && e.ok()) {
+    wide_energy_out_kernel<<<1, 32, 0, s>>>(e.slots, sq_err);
+    e.check_launch("wide_energy_out_kernel launch");
+  }
+  if (what) *what = e.what;
+  return e.err;
+}
+
+}  // namespace
+
+cudaError_t wide_density_grid(cudaStream_t s, const FlowLayout& lay, const SplineConsts<float>& sc, const float* weights,
+                              const float* t_host, int n_t, double x_min, double x_step, double y_min, double y_step, int nx,
+                              int ny, float* density, int with_ref, float mix, float var0, float var1, double* sq_err,
+                              void* workspace, const char** what) {
+  DensityPoints dp = {};
+  dp.mode = 0; dp.nx = nx; dp.ny = ny;
+  dp.x_min = x_min; dp.x_step = x_step; dp.y_min = y_min; dp.y_step = y_step;
+  // the times follow the chunk buffers in the workspace
+  float* t_dev = (float*)((char*)workspace + carve(nullptr, lay, chunk_rows(), false, 1, nullptr));
+  cudaError_t err = cudaMemcpyAsync(t_dev, t_host, (size_t)n_t * sizeof(float), cudaMemcpyHostToDevice, s);
+  if (err != cudaSuccess) {
+    if (what) *what = "H2D times";
+    return err;
+  }
+  dp.t_dev = t_dev;
+  return run_density(s, lay, sc, weights, dp, (int64_t)nx * ny * n_t, nullptr, density, with_ref, mix, var0, var1, sq_err,
+                     workspace, what);
+}
+
+cudaError_t wide_density_mc(cudaStream_t s, const FlowLayout& lay, const SplineConsts<float>& sc, const float* weights,
+                            float cond, uint64_t key_n, uint32_t step, int64_t n, float* samples, float* density,
+                            int with_ref, float mix, float var0, float var1, double* sq_err, void* workspace,
+                            const char** what) {
+  DensityPoints dp = {};
+  dp.mode = 1; dp.key_n = key_n; dp.step = step; dp.cond = cond;
+  return run_density(s, lay, sc, weights, dp, n, samples, density, with_ref, mix, var0, var1, sq_err, workspace, what);
 }
 
 }  // namespace cnfot

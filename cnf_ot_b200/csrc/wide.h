@@ -35,4 +35,21 @@ cudaError_t wide_kinetic_energy(cudaStream_t s, const FlowLayout& lay, const Spl
                                 const float* latent, int64_t batch, int latent_blocks, const float* t_host, int n_t, float dt,
                                 int with_score, float kappa, float dx, double* out, void* workspace, const char** what);
 
+// cnfot_density_grid / cnfot_density_mc (density_kernel of flow_kernels.cuh), chunk by chunk: density = exp(log_prob) of
+// every point (may be NULL) and, with_ref, the summed squared error against (1 - mix) N(0, var0 I) + mix N(0, var1 I)
+// into sq_err (one double on the device).  Workspace: the chunk buffers (independent of the number of points) and the
+// n_t grid times.
+int64_t wide_density_workspace_bytes(const FlowLayout& lay, int n_t);
+// grid: the nx x ny points (x_min + ix x_step, y_min + iy y_step) at each of the n_t times, density[(ti, iy, ix)]
+cudaError_t wide_density_grid(cudaStream_t s, const FlowLayout& lay, const SplineConsts<float>& sc, const float* weights,
+                              const float* t_host, int n_t, double x_min, double x_step, double y_min, double y_step, int nx,
+                              int ny, float* density, int with_ref, float mix, float var0, float var1, double* sq_err,
+                              void* workspace, const char** what);
+// Monte-Carlo: samples (n x D, may be NULL) and densities of sample_and_log_prob at time `cond` for rows [0, n) of the
+// NORMAL (n, D) draw of (key_n = key ^ philox_salt(kDrawNormal, n), step)
+cudaError_t wide_density_mc(cudaStream_t s, const FlowLayout& lay, const SplineConsts<float>& sc, const float* weights,
+                            float cond, uint64_t key_n, uint32_t step, int64_t n, float* samples, float* density,
+                            int with_ref, float mix, float var0, float var1, double* sq_err, void* workspace,
+                            const char** what);
+
 }  // namespace cnfot

@@ -471,7 +471,7 @@ def kinetic_energy(shape: FlowShape, weights, latent, t_values: Sequence[float],
 def density_grid(shape: FlowShape, weights, t_values: Sequence[float], domain, nx: int, ny: int, ref=None,
                  want_density: bool = True):
   """exp(log_prob) on the grid hstack(meshgrid(linspace(x0, x1, nx), linspace(y0, y1, ny))) for every time of `t_values`
-  in ONE kernel launch (cnfot_density_grid).  domain = (x0, x1, y0, y1).  ref = (mix, var0, var1): also the sum of squared
+  in ONE kernel launch (cnfot_density_grid; wide flows: one flow pass per row chunk).  domain = (x0, x1, y0, y1).  ref = (mix, var0, var1): also the sum of squared
   errors against (1 - mix) N(0, var0 I) + mix N(0, var1 I).  Returns (density (n_t, ny, nx) or None, sq_err 0-d float64 or None)."""
   lib = _lib.load()
   weights = _dev(weights, "weights")

@@ -65,7 +65,8 @@ def calc_score_kinetic_energy(sample_fn, log_prob_fn, params, T: float = 1, beta
 
 # ------------------------------------------------------------------ densities on grids / at samples (SURVEY.md §8f row 3)
 # The numerical content of the reference's plotting helpers and of the fp evaluation tail, without matplotlib:
-# each is ONE kernel launch (cnfot_density_grid / cnfot_density_mc), the grid generated on chip.
+# each is ONE kernel launch (cnfot_density_grid / cnfot_density_mc; wide flows: one flow pass per row chunk on the
+# wide-conditioner engine), the grid generated on chip.
 def _model_of_fn(fn):
   model = getattr(fn, "__self__", None)
   if model is None or not hasattr(model, "shape"):

@@ -337,7 +337,11 @@ CNFOT_API int cnfot_kinetic_energy(void* stream, const cnfot_flow_desc* flow, co
  *                       (solvers.py:254-278).  samples: (n, dim) or NULL; density: (n) exp(log_prob) or NULL.
  * with_ref != 0: *sq_err (ONE double on the device) = sum over the points of
  *   (density - ((1 - mix) N(y; 0, var0 I) + mix N(y; 0, var1 I)))^2       (solvers.py:238-252,270-276,296-299);
- * the caller takes sqrt(sq_err / points). */
+ * the caller takes sqrt(sq_err / points).
+ * Both engines run these calls: the fused kernels in one launch, flows with wide conditioners chunk by chunk on the
+ * wide-conditioner engine (cnfot_last_launch_info reports engine 4).  Workspace: for the fused kernels the per-CTA
+ * partial sums and the n_t times; for wide flows the chunk buffers of one flow pass and the n_t times -- independent of
+ * the number of points (n_t = 0 for cnfot_density_mc). */
 CNFOT_API int64_t cnfot_density_workspace_bytes(const cnfot_flow_desc* flow, int32_t n_t);
 CNFOT_API int cnfot_density_grid(void* stream, const cnfot_flow_desc* flow, const float* weights, const float* t_host,
                        int32_t n_t, double x_min, double x_max, double y_min, double y_max, int32_t nx, int32_t ny,
