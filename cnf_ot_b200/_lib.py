@@ -76,6 +76,7 @@ SIGNATURES = {
   "cnfot_abi_version": (c_int32, []),
   "cnfot_last_error": (c_char_p, []),
   "cnfot_last_launch_info": (None, [POINTER(c_int32)] * 4),
+  "cnfot_last_launch_variant": (None, [POINTER(c_int32)] * 4),
   "cnfot_debug_step_timeline": (None, [c_void_p]),
   "cnfot_workspace_register": (c_int32, [c_void_p, _F, c_void_p, c_int64]),
   "cnfot_workspace_release": (c_int32, [c_void_p]),
@@ -169,6 +170,14 @@ def last_launch_info() -> dict:
   eng = vals[3].value  # 0 CUDA cores, 1 tcgen05 engine, 2 warp-level MMA engine, 4 wide-conditioner engine
   return {"grid": vals[0].value, "smem_bytes": vals[1].value, "ctas_per_sm": vals[2].value,
           "tensor_cores": bool(eng), "engine": {0: "cuda", 1: "tc", 2: "mma", 4: "wide"}.get(eng, "?")}
+
+
+def last_launch_variant() -> dict:
+  """Kernel instantiation of the calling thread's most recent fused step / VJP launch (cnfot_last_launch_variant)."""
+  vals = [c_int32(0) for _ in range(4)]
+  load().cnfot_last_launch_variant(*[ctypes.byref(v) for v in vals])
+  plan = {0: "cuda", 1: "tc", 2: "mma", 3: "mma_stream", 4: "wide"}.get(vals[0].value, None)
+  return {"plan": plan, "stash_tmem_cols": vals[1].value, "kinetic_group": vals[2].value, "latency": bool(vals[3].value)}
 
 
 def check(rc: int) -> None:

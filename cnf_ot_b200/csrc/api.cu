@@ -139,6 +139,14 @@ struct LaunchCfg {
   size_t smem;
 };
 static thread_local int g_last_launch[4] = {0, 0, 0, 0};
+// cnfot_last_launch_variant: {plan, stash TMEM columns, kinetic lane group, latency instantiation} of the most recent
+// fused call.  The step and VJP entries reset it on entry and fill it in once their kernel is chosen; every other fused
+// launch resets it (configure(), the wide-engine evaluation, energy and density paths).  Plan -1: not a step or VJP.
+static thread_local int g_last_variant[4] = {-1, 0, 0, 0};
+static void record_variant(int plan, int stash_cols, int kinetic_group, bool latency) {
+  g_last_variant[0] = plan; g_last_variant[1] = stash_cols; g_last_variant[2] = kinetic_group;
+  g_last_variant[3] = latency ? 1 : 0;
+}
 
 // Shared-memory plan and engine choice.
 //   warp-MMA engine (warp_mlp.cuh)  16-wide networks: the default there.  Weights + hi/lo fragments resident
@@ -247,6 +255,7 @@ static int configure(const void* kernel, const SmemPlan& sp, int64_t tiles, Laun
   g_last_launch[1] = (int)smem;
   g_last_launch[2] = occ;
   g_last_launch[3] = sp.off_wmma >= 0 ? kEngTc : (sp.off_frag >= 0 ? kEngMma : kEngCuda);  // 2 also for the streamed plan
+  record_variant(-1, 0, 0, false);
   return 0;
 }
 
@@ -436,6 +445,12 @@ void cnfot_last_launch_info(int32_t* grid, int32_t* smem_bytes, int32_t* ctas_pe
   if (ctas_per_sm) *ctas_per_sm = g_last_launch[2];
   if (tensor_cores) *tensor_cores = g_last_launch[3];
 }
+void cnfot_last_launch_variant(int32_t* plan, int32_t* stash_tmem_cols, int32_t* kinetic_group, int32_t* latency) {
+  if (plan) *plan = g_last_variant[0];
+  if (stash_tmem_cols) *stash_tmem_cols = g_last_variant[1];
+  if (kinetic_group) *kinetic_group = g_last_variant[2];
+  if (latency) *latency = g_last_variant[3];
+}
 const char* cnfot_last_error(void) { return g_err; }
 
 int64_t cnfot_param_count(const cnfot_flow_desc* flow) {
@@ -569,6 +584,7 @@ static int flow_eval_call(int dir, void* stream, const cnfot_flow_desc* flow, co
                                    rows, out, logdet, add_base, workspace, &what);
     if (e != cudaSuccess) return cuda_fail(e, what);
     g_last_launch[0] = 0; g_last_launch[1] = 0; g_last_launch[2] = 0; g_last_launch[3] = kEngWide;
+    record_variant(-1, 0, 0, false);
     return 0;
   }
   if (int rc = check_fused(flow, lay)) return rc;
@@ -632,6 +648,7 @@ static int flow_vjp_call(int dir, void* stream, const cnfot_flow_desc* flow, con
                          const float* in, const float* cond, int64_t cond_stride, int64_t rows,
                          const float* g_out, const float* g_logdet, int32_t add_base, float* g_in,
                          float* g_weights, void* workspace, int64_t workspace_bytes) {
+  record_variant(-1, 0, 0, false);   // a call that launches no VJP kernel (rows == 0, errors) leaves no variant behind
   FlowLayout lay;
   if (int rc = check_flow(flow, &lay)) return rc;
   if (use_wide(flow, lay)) {
@@ -647,6 +664,7 @@ static int flow_vjp_call(int dir, void* stream, const cnfot_flow_desc* flow, con
                                   rows, g_out, g_logdet, add_base, g_in, g_weights, workspace, &what);
     if (e != cudaSuccess) return cuda_fail(e, what);
     g_last_launch[0] = 0; g_last_launch[1] = 0; g_last_launch[2] = 0; g_last_launch[3] = kEngWide;
+    record_variant(kEngWide, 0, 0, false);
     return 0;
   }
   if (int rc = check_fused(flow, lay)) return rc;
@@ -669,6 +687,7 @@ static int flow_vjp_call(int dir, void* stream, const cnfot_flow_desc* flow, con
   const void* kernel = find_flow_vjp_kernel(lay, engine, stash_cols > 0);
   LaunchCfg cfg;
   if (int rc = configure(kernel, sp, (rows + kTile - 1) / kTile, &cfg, stash_cols)) return rc;
+  record_variant(engine, stash_cols, 0, false);
   unsigned long long* counter;
   VjpArgs a;
   a.W = weights; a.frags = nullptr; a.in = in; a.cond = cond; a.cond_stride = cond_stride; a.rows = rows;
@@ -792,6 +811,7 @@ static int mfc_step_wide(void* stream, const cnfot_flow_desc* flow, const FlowLa
                                 t_batch_host, n_t, rows_B, rows_b, out, workspace, &what);
   if (e != cudaSuccess) return cuda_fail(e, what);
   g_last_launch[0] = 0; g_last_launch[1] = 0; g_last_launch[2] = 0; g_last_launch[3] = kEngWide;
+  record_variant(kEngWide, 0, 0, false);
   return 0;
 }
 
@@ -835,6 +855,7 @@ static int mfc_step_impl(void* stream, const cnfot_flow_desc* flow, const cnfot_
                          const float* weights, const StepIo& io, int32_t n_t,
                          int64_t rows_B, int64_t rows_b, int64_t global_B, int64_t global_b, float lambda,
                          void* workspace, int64_t workspace_bytes) {
+  record_variant(-1, 0, 0, false);   // a call that launches no step kernel (no rows, errors) leaves no variant behind
   FlowLayout lay;
   if (int rc = check_flow(flow, &lay)) return rc;
   if (use_wide(flow, lay)) {
@@ -954,6 +975,7 @@ static int mfc_step_impl(void* stream, const cnfot_flow_desc* flow, const cnfot_
   a.salt_t = philox_salt(kDrawUniform, (uint64_t)n_t);
   LaunchCfg cfg;
   if (int rc = configure(kernel, sp, (tiles * unit + kTile - 1) / kTile, &cfg, stash_cols)) return rc;
+  record_variant(engine, stash_cols, group, engine == kEngMmaStream && group == 1 && latency);
   a.W = weights;
   a.frags = nullptr;
   if (engine == kEngMmaStream) {
@@ -1375,6 +1397,7 @@ int cnfot_kinetic_energy(void* stream, const cnfot_flow_desc* flow, const float*
                                          latent_blocks, t_host, n_t, dt, with_score, kappa, dx, out, workspace, &what);
     if (we != cudaSuccess) return cuda_fail(we, what);
     g_last_launch[0] = 0; g_last_launch[1] = 0; g_last_launch[2] = 0; g_last_launch[3] = kEngWide;
+    record_variant(-1, 0, 0, false);
     return 0;
   }
   cudaStream_t s = (cudaStream_t)stream;
@@ -1448,6 +1471,7 @@ static int density_call(void* stream, const cnfot_flow_desc* flow, const float* 
                           a.with_ref, a.mix, a.var0, a.var1, sq_err, workspace, &what);
     if (we != cudaSuccess) return cuda_fail(we, what);
     g_last_launch[0] = 0; g_last_launch[1] = 0; g_last_launch[2] = 0; g_last_launch[3] = kEngWide;
+    record_variant(-1, 0, 0, false);
     return 0;
   }
   float* t_dev = (float*)((char*)workspace + partial_bytes(lay));

@@ -91,6 +91,15 @@ CNFOT_API const char* cnfot_last_error(void);
  * GEMMs, the other three fields are 0). */
 CNFOT_API void cnfot_last_launch_info(int32_t* grid, int32_t* smem_bytes, int32_t* ctas_per_sm,
                                       int32_t* tensor_cores);
+/* Kernel instantiation of the calling thread's most recent fused call, when that call was a step or a VJP that
+ * launched its kernel (diagnostics, tests).  plan: 0 CUDA cores, 1 tcgen05 engine, 2 warp-level tensor-core engine with
+ * weights resident in shared memory, 3 the same streaming weights from the workspace, 4 wide-conditioner engine; -1 the
+ * most recent call was another fused call (evaluation, energies, densities, on either engine), or a step or VJP that
+ * launched no kernel (no rows, an argument error).  stash_tmem_cols: TMEM columns per CTA of the activation stash,
+ * 0 = the backward pass recomputes.  kinetic_group: lanes per kinetic row of a step (1 = one thread per row), 0 for
+ * anything but a step.  latency: 1 = the two-CTAs-per-SM instantiation of the streamed plan. */
+CNFOT_API void cnfot_last_launch_variant(int32_t* plan, int32_t* stash_tmem_cols, int32_t* kinetic_group,
+                                         int32_t* latency);
 /* Diagnostics (tools/step_timeline.py): while `device_words` is non-NULL (8 uint64 in device memory, initialised by the
  * caller to {~0, 0, ~0, 0, 0, 0, 0, 0}) every fused train step records %globaltimer stamps there: [0] first CTA starts,
  * [1] last CTA finished its setup, [2] / [3] first / last CTA ran out of row tiles, [4] last CTA enters the
