@@ -416,6 +416,149 @@ CNFOT_CALL void flow_pass_bwd(const DimsT& dm, const SC& sc, T t, const T* state
   }
 }
 
+// ---- the log-prob pass of the 2-D, 2-layer flow on the stash engine, unrolled ------------------------------------
+// flow_pass / flow_pass_bwd are real calls with rolled loops: the row's states, its adjoint, the context, the shape and
+// the knot adjoints of `first` reach them by reference and live in local memory.  For Dims<2, 2> the whole pass is known
+// at compile time -- position 0 of a layer is always the `first` spline, position 1 always the conditioner, and layer l
+// handles coordinate l & 1 first (perm_at) -- so the pair below is flow_pass<1> / flow_pass_bwd<1> inlined into the row,
+// with the states as named scalars and the knot adjoints in registers (what still goes to local memory is the register
+// allocator's spill code).  Only row_nll uses it (the log-prob rows: 97 % of the rows of an ot step), and only in the
+// kernels with the activation stash (Ctx::kStash).  Measured on B200 (DESIGN 4.2): with the sample rows inlined as well,
+// or in the recompute kernels, the extra live values spill and cost more than the calls.
+template <class Ctx, bool = Ctx::kWarpMlp>
+struct CtxHasStash { static constexpr bool value = false; };
+template <class Ctx>
+struct CtxHasStash<Ctx, true> { static constexpr bool value = Ctx::kStash; };
+template <class DimsT, class Ctx>
+constexpr bool kFlow2dInline = DimsT::kD == 2 && DimsT::kL == 2 && CtxHasStash<Ctx>::value;
+
+// the three states of a pass: its input, the result of step 0, the result of step 1 (flow_pass: states[0..6))
+template <typename T>
+struct Pass2d {
+  T in0, in1, mid0, mid1, out0, out1;
+};
+
+// the entries of a FirstGrad that first_grad_to_raw reads
+template <typename T, int K>
+CNFOT_HD void first_grad_copy(FirstGrad<T, K>& dst, const FirstGrad<T, K>& src) {
+#pragma unroll
+  for (int k = 0; k <= K; ++k) {
+    if (k >= 1 && k < K) { dst.gx[k] = src.gx[k]; dst.gy[k] = src.gy[k]; }
+    dst.gd[k] = src.gd[k];
+  }
+}
+
+// first_grad_add with compile-time indices, so that `a` can live in registers: every entry takes its term or zero
+// (x + 0 == x: the same sums).  Entries 0 and K of gx and gy are never read (first_grad_to_raw) and are left alone.
+template <typename T, int K>
+CNFOT_HD void first_grad_add_unrolled(FirstGrad<T, K>& a, const SplineState<T, K>& st, const KnotAdjoints<T>& ka) {
+  const bool in = st.tail == 0;
+#pragma unroll
+  for (int k = 0; k <= K; ++k) {
+    const bool lo = in && st.idx == k, hi = in && st.idx + 1 == k;
+    if (k >= 1 && k < K) {
+      a.gx[k] += lo ? ka.gx0 : (hi ? ka.gx1 : (T)0);
+      a.gy[k] += lo ? ka.gy0 : (hi ? ka.gy1 : (T)0);
+    }
+    const bool tail = (k == 0 && st.tail == 1) || (k == K && st.tail == 2);
+    a.gd[k] += lo ? ka.gd0 : (hi ? ka.gd1 : (tail ? ka.gst : (T)0));
+  }
+}
+
+// Step S of flow_pass<1> (layer 1 - S): (v0, v1) -> (u0, u1), the log-dets added to ld_total in flow_pass's order.
+template <int S, typename T, class Net, class Ctx, class SC>
+CNFOT_HD void flow_step_2d(const SC& sc, T t, T v0, T v1, T& u0, T& u1, T& ld_total, Ctx& ctx, bool stash) {
+  constexpr int K = Net::kK, Pp = Net::kPp;
+  constexpr int layer = 1 - S;
+  constexpr bool swap = (layer & 1) != 0;   // position 0 handles coordinate perm_at(layer, 0, 2) = layer & 1
+  const T va = swap ? v1 : v0, vb = swap ? v0 : v1;
+  T ua, ub, ld;
+  {
+    SplineState<T, K> st;
+    rqs_locate_first<false, T, K>(va, ctx.first_knots(), sc, st);
+    rqs_forward_map<T, K>(va, st, sc, ua, ld);
+    ld_total += ld;
+  }
+  {
+    // the conditioner reads cvec[perm_at(layer, 0, 2)] only: the output of position 0
+    const T cv[2] = {ua, ua};
+    T theta[Pp];
+    ctx.cond_forward(2, layer, 1, t, cv, theta, false, stash);
+    SplineState<T, K> st;
+    rqs_locate_raw<false, T, K>(vb, theta, sc, st);
+    if (stash) ctx.stash_state(2, layer, 1, st);
+    rqs_forward_map<T, K>(vb, st, sc, ub, ld);
+    ld_total += ld;
+  }
+  u0 = swap ? ub : ua;
+  u1 = swap ? ua : ub;
+}
+
+// flow_pass<1> for Dims<2, 2>: p.in0, p.in1 are the input; fills the other states, returns the summed log-det.
+template <typename T, class Net, class Ctx, class SC>
+CNFOT_HD T flow_pass_2d(const SC& sc, T t, Pass2d<T>& p, Ctx& ctx, bool stash) {
+  T ld_total = (T)0;
+  flow_step_2d<0, T, Net>(sc, t, p.in0, p.in1, p.mid0, p.mid1, ld_total, ctx, stash);
+  flow_step_2d<1, T, Net>(sc, t, p.mid0, p.mid1, p.out0, p.out1, ld_total, ctx, stash);
+  return ld_total;
+}
+
+// Reverse mode of step S: (g0, g1) from the adjoint of its output (u0, u1) to that of its input (v0, v1).
+// Position 1 first, so that the adjoint of position 0's coordinate is complete before position 0 reads it.
+template <int S, typename T, class Net, class Ctx, class SC>
+CNFOT_HD void flow_step_bwd_2d(const SC& sc, T t, T v0, T v1, T u0, T u1, T& g0, T& g1, T gld,
+                               FirstGrad<T, Net::kK>& gfirst, Ctx& ctx, bool stash) {
+  constexpr int K = Net::kK, Pp = Net::kPp;
+  constexpr int layer = 1 - S;
+  constexpr bool swap = (layer & 1) != 0;
+  const T va = swap ? v1 : v0, vb = swap ? v0 : v1;
+  const T ua = swap ? u1 : u0;   // the conditioner's input
+  T ga = swap ? g1 : g0, gb = swap ? g0 : g1;
+  {
+    const T cv[2] = {ua, ua};
+    SplineState<T, K> st;
+    if (stash) {
+      ctx.cond_restore(2, layer, 1, st, sc.min_slope);
+    } else {
+      T theta[Pp];
+      ctx.cond_forward(2, layer, 1, t, cv, theta, true);
+      rqs_locate_raw<false, T, K>(vb, theta, sc, st);
+    }
+    KnotAdjoints<T> ka;
+    gb = rqs_forward_map_bwd<T, K>(vb, st, sc, gb, gld, ka);
+    T gtheta[Pp];
+#pragma unroll
+    for (int j = 0; j < Pp; ++j) gtheta[j] = (T)0;
+    scatter_to_raw<T, K>(st, sc, ka.gx0, ka.gx1, ka.gy0, ka.gy1, ka.gd0, ka.gd1, ka.gst, gtheta);
+    // the engine adds the adjoint of its input to gvec[perm_at(layer, 0, 2)]
+    T gv[2] = {ga, ga};
+    ctx.cond_backward(2, layer, 1, t, cv, gtheta, gv);
+    ga = swap ? gv[1] : gv[0];
+  }
+  {
+    SplineState<T, K> st;
+    rqs_locate_first<false, T, K>(va, ctx.first_knots(), sc, st);
+    KnotAdjoints<T> ka;
+    ga = rqs_forward_map_bwd<T, K>(va, st, sc, ga, gld, ka);
+    first_grad_add_unrolled<T, K>(gfirst, st, ka);
+  }
+  g0 = swap ? gb : ga;
+  g1 = swap ? ga : gb;
+}
+
+// flow_pass_bwd<1> for Dims<2, 2> on the states flow_pass_2d left in p: (g0, g1) from the adjoint of p.out to that of
+// p.in.  The knot adjoints of `first` are added to gfirst in the order flow_pass_bwd adds them, through a copy in
+// registers that lives for this pass only.
+template <typename T, class Net, class Ctx, class SC>
+CNFOT_HD void flow_pass_bwd_2d(const SC& sc, T t, const Pass2d<T>& p, T& g0, T& g1, T gld, FirstGrad<T, Net::kK>& gfirst,
+                               Ctx& ctx, bool stash) {
+  FirstGrad<T, Net::kK> acc;
+  first_grad_copy<T, Net::kK>(acc, gfirst);
+  flow_step_bwd_2d<1, T, Net>(sc, t, p.mid0, p.mid1, p.out0, p.out1, g0, g1, gld, acc, ctx, stash);
+  flow_step_bwd_2d<0, T, Net>(sc, t, p.in0, p.in1, p.mid0, p.mid1, g0, g1, gld, acc, ctx, stash);
+  first_grad_copy<T, Net::kK>(gfirst, acc);
+}
+
 // log N(x; 0, I)
 template <typename T>
 CNFOT_HD T base_log_prob(const T* x, int D) {

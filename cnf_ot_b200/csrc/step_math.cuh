@@ -120,16 +120,29 @@ template <typename T, class Net, class DimsT, class Ctx, class SC, class FG>
 CNFOT_HD T row_nll(const DimsT& dm, const SC& sc, T t, const T* data, T weight,
                    FG& gfirst, const RowTiles<T, Net>& tl, Ctx& ctx) {
   const int D = dm.D(), L = dm.L();
-  T st[kMaxStateFloats];
-  for (int i = 0; i < D; ++i) st[i] = data[i];
-  const bool stash = ctx.stash_on();   // forward and backward of the same rows, back to back: keep the activations
-  T ld = flow_pass<1, T, Net, DimsT, Ctx>(dm, sc, t, st, tl, ctx, stash);
-  const T* x = st + L * D;
-  T lp = base_log_prob<T>(x, D) + ld;
-  T g[kMaxDim];
-  for (int i = 0; i < D; ++i) g[i] = weight * x[i];  // d(-w lp)/dx = w x
-  flow_pass_bwd<1, T, Net, DimsT, Ctx>(dm, sc, t, st, g, -weight, gfirst, tl, ctx, stash);
-  return -weight * lp;
+  if constexpr (kFlow2dInline<DimsT, Ctx>) {
+    const bool stash = ctx.stash_on();
+    Pass2d<T> p;
+    p.in0 = data[0];
+    p.in1 = data[1];
+    const T ld = flow_pass_2d<T, Net>(sc, t, p, ctx, stash);
+    const T x[2] = {p.out0, p.out1};
+    const T lp = base_log_prob<T>(x, 2) + ld;
+    T g0 = weight * p.out0, g1 = weight * p.out1;
+    flow_pass_bwd_2d<T, Net>(sc, t, p, g0, g1, -weight, gfirst, ctx, stash);
+    return -weight * lp;
+  } else {
+    T st[kMaxStateFloats];
+    for (int i = 0; i < D; ++i) st[i] = data[i];
+    const bool stash = ctx.stash_on();   // forward and backward of the same rows, back to back: keep the activations
+    T ld = flow_pass<1, T, Net, DimsT, Ctx>(dm, sc, t, st, tl, ctx, stash);
+    const T* x = st + L * D;
+    T lp = base_log_prob<T>(x, D) + ld;
+    T g[kMaxDim];
+    for (int i = 0; i < D; ++i) g[i] = weight * x[i];  // d(-w lp)/dx = w x
+    flow_pass_bwd<1, T, Net, DimsT, Ctx>(dm, sc, t, st, g, -weight, gfirst, tl, ctx, stash);
+    return -weight * lp;
+  }
 }
 
 // ---- rows pushed through the sample direction at one time t ----------------------

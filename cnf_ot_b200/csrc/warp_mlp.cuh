@@ -268,6 +268,7 @@ struct DeviceCtxMma {
     else return s_wt;
   }
   static constexpr bool kWarpMlp = true;
+  static constexpr bool kStash = STASH;   // the activation stash is compiled in (kEngMmaStash)
   static constexpr bool kAccInGlobal = true;
   static constexpr int H = Net::kH, M = Net::kM, Pp = Net::kPp;
   static_assert(H == 16 && Pp == 16, "the warp-MMA engine is written for 16-wide layers");
