@@ -118,6 +118,7 @@ SIGNATURES = {
   "cnfot_mfc_step_rng_host": (c_int32, [c_void_p, _F, _P, c_void_p, ctypes.c_uint64, ctypes.c_uint32, c_int32, c_int64,
                                         c_int64, c_int64, c_int64, c_int64, c_int64, c_float, c_void_p, c_void_p, c_int64]),
   "cnfot_train_state_bytes": (c_int64, [_F]),
+  "cnfot_train_state_bytes_rows": (c_int64, [_F, c_int64, c_int64]),
   "cnfot_train_state_init": (c_int32, [c_void_p, _F, c_void_p, c_int64, ctypes.c_uint64, ctypes.c_uint64, ctypes.c_uint32]),
   "cnfot_mfc_update": (c_int32, [c_void_p, _F, _P, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, POINTER(AdamDesc),
                                  c_int32, c_int64, c_int64, c_int64, c_int64, c_int64, c_int64, c_float, c_void_p,

@@ -778,41 +778,10 @@ int64_t cnfot_mfc_step_workspace_bytes(const cnfot_flow_desc* flow, int64_t rows
   return step_ws_bytes(flow, lay, rows_B, rows_b);
 }
 
-// The step on the wide-conditioner engine (wide.cu): hidden >= 64, e.g. BASELINE config 5.
-static int mfc_step_wide(void* stream, const cnfot_flow_desc* flow, const FlowLayout& lay,
-                         const cnfot_problem_desc* problem, const float* weights, const float* latent, const float* latent_sub,
-                         const float* src, const float* tgt, const float* t_batch_host, int32_t n_t, int64_t rows_B,
-                         int64_t rows_b, int64_t global_B, int64_t global_b, float lambda, float* out, void* workspace,
-                         int64_t workspace_bytes, bool accumulate, const cnfot_peer_desc* peers) {
-  if (!problem) return fail(CNFOT_ERR_ARG, "problem descriptor is NULL");
-  if (peers)
-    return fail(CNFOT_ERR_ARG, "the wide-conditioner engine has no fused all-reduce (its gradient is hundreds of MB): "
-                               "call cnfot_mfc_step and all-reduce `out` with NCCL");
-  if (accumulate) return fail(CNFOT_ERR_ARG, "the wide-conditioner engine does not take chunked host input");
-  if (rows_B < 0 || rows_b < 0 || global_B < 1 || global_b < 1 || rows_B > global_B || rows_b > global_b)
-    return fail(CNFOT_ERR_ARG, "bad row counts");
-  if (n_t < 1) return fail(CNFOT_ERR_ARG, "t_batch_size must be >= 1");
-  if (!weights || !out || !workspace || !t_batch_host) return fail(CNFOT_ERR_ARG, "NULL buffer");
-  if (problem->type == CNFOT_OT) {
-    if (rows_B > 0 && (!src || !tgt)) return fail(CNFOT_ERR_ARG, "ot needs src and tgt batches");
-  } else if (rows_B > 0 && !latent) {
-    return fail(CNFOT_ERR_ARG, "latent is NULL");
-  }
-  if (rows_b > 0 && !latent_sub) return fail(CNFOT_ERR_ARG, "latent_sub is NULL");
-  const int64_t need = wide_step_workspace_bytes(lay, rows_B, rows_b);
-  if (workspace_bytes < need) return fail(CNFOT_ERR_WORKSPACE, "workspace too small: %lld < %lld",
-                                          (long long)workspace_bytes, (long long)need);
-  StepConsts<float> pc;
-  const char* err = nullptr;
-  if (make_step_consts<float>(*problem, lay.D, (double)lambda, global_B, global_b, n_t, &pc, &err))
-    return fail(CNFOT_ERR_ARG, "%s", err);
-  const char* what = "";
-  cudaError_t e = wide_mfc_step((cudaStream_t)stream, lay, spline_consts(flow), pc, weights, latent, latent_sub, src, tgt,
-                                t_batch_host, n_t, rows_B, rows_b, out, workspace, &what);
-  if (e != cudaSuccess) return cuda_fail(e, what);
-  g_last_launch[0] = 0; g_last_launch[1] = 0; g_last_launch[2] = 0; g_last_launch[3] = kEngWide;
-  record_variant(kEngWide, 0, 0, false);
-  return 0;
+// train state of a wide flow: [header (kCounterBytes: the state words) | gradient + loss slots | step workspace]
+static int64_t wide_grad_bytes(const FlowLayout& lay) { return ((int64_t)(lay.total + kNumSlots) * (int64_t)sizeof(float) + 255) / 256 * 256; }
+static int64_t wide_train_state_bytes(const FlowLayout& lay, int64_t rows_B, int64_t rows_b) {
+  return kCounterBytes + wide_grad_bytes(lay) + wide_step_workspace_bytes(lay, rows_B, rows_b);
 }
 
 // Everything a step call can vary: where the rows come from, what the kernel's tail does with the result.
@@ -842,6 +811,71 @@ struct StepIo {
   int64_t loss_hist_len = 0;
 };
 
+// The step on the wide-conditioner engine (wide.cu): hidden >= 64, e.g. BASELINE config 5.  Explicit rows, on-chip
+// draws and the device-resident update (io.stateful: `workspace` is the train state, wide_train_state_bytes)
+static int mfc_step_wide(void* stream, const cnfot_flow_desc* flow, const FlowLayout& lay,
+                         const cnfot_problem_desc* problem, const float* weights, const StepIo& io, int32_t n_t,
+                         int64_t rows_B, int64_t rows_b, int64_t global_B, int64_t global_b, float lambda, void* workspace,
+                         int64_t workspace_bytes) {
+  if (!problem) return fail(CNFOT_ERR_ARG, "problem descriptor is NULL");
+  if (io.peers)
+    return fail(CNFOT_ERR_ARG, "the wide-conditioner engine has no fused all-reduce (its gradient is hundreds of MB): "
+                               "call cnfot_mfc_step and all-reduce `out` with NCCL");
+  if (io.accumulate) return fail(CNFOT_ERR_ARG, "the wide-conditioner engine does not take chunked host input");
+  if (rows_B < 0 || rows_b < 0 || global_B < 1 || global_b < 1 || rows_B > global_B || rows_b > global_b)
+    return fail(CNFOT_ERR_ARG, "bad row counts");
+  if (n_t < 1) return fail(CNFOT_ERR_ARG, "t_batch_size must be >= 1");
+  if (!weights || !workspace || (!io.out && !io.stateful)) return fail(CNFOT_ERR_ARG, "NULL buffer");
+  if (!io.rng) {
+    if (!io.t_batch_host) return fail(CNFOT_ERR_ARG, "NULL buffer");
+    if (problem->type == CNFOT_OT) {
+      if (rows_B > 0 && (!io.src || !io.tgt)) return fail(CNFOT_ERR_ARG, "ot needs src and tgt batches");
+    } else if (rows_B > 0 && !io.latent) {
+      return fail(CNFOT_ERR_ARG, "latent is NULL");
+    }
+    if (rows_b > 0 && !io.latent_sub) return fail(CNFOT_ERR_ARG, "latent_sub is NULL");
+  } else if (io.row0_B < 0 || io.row0_b < 0 || io.row0_B + rows_B > global_B || io.row0_b + rows_b > global_b) {
+    return fail(CNFOT_ERR_ARG, "shard [row0, row0 + rows) outside the global batch");
+  }
+  const int64_t need = io.stateful ? wide_train_state_bytes(lay, rows_B, rows_b) : wide_step_workspace_bytes(lay, rows_B, rows_b);
+  if (workspace_bytes < need)
+    return fail(CNFOT_ERR_WORKSPACE, "%s too small: %lld < %lld", io.stateful ? "train state" : "workspace",
+                (long long)workspace_bytes, (long long)need);
+  StepConsts<float> pc;
+  const char* err = nullptr;
+  if (make_step_consts<float>(*problem, lay.D, (double)lambda, global_B, global_b, n_t, &pc, &err))
+    return fail(CNFOT_ERR_ARG, "%s", err);
+  WideDraws dr = {};
+  WideAdam adam = {};
+  float* out = io.out;
+  void* ws = workspace;
+  if (io.rng) {
+    dr.key = io.key; dr.step = io.step;
+    dr.salts = step_salts(global_B, global_b, n_t);
+    dr.row0_B = io.row0_B; dr.row0_b = io.row0_b;
+  }
+  if (io.stateful) {
+    // train state: [header (key, step, epoch at kStateWordOffset) | gradient + loss slots | step workspace]
+    char* base = (char*)workspace;
+    unsigned long long* words = (unsigned long long*)base + kStateWordOffset;
+    dr.state = words;
+    adam.state = words;
+    adam.weights = io.weights_rw; adam.m = io.adam_m; adam.v = io.adam_v;
+    adam.lr = io.lr; adam.b1 = io.b1; adam.b2 = io.b2; adam.eps = io.eps;
+    adam.loss_hist = io.loss_hist; adam.loss_hist_len = io.loss_hist_len;
+    if (!out) out = (float*)(base + kCounterBytes);
+    ws = base + kCounterBytes + wide_grad_bytes(lay);
+  }
+  const char* what = "";
+  cudaError_t e = wide_mfc_step((cudaStream_t)stream, lay, spline_consts(flow), pc, weights, io.latent, io.latent_sub, io.src,
+                                io.tgt, io.t_batch_host, io.rng ? &dr : nullptr, n_t, rows_B, rows_b, out,
+                                io.stateful ? &adam : nullptr, ws, &what);
+  if (e != cudaSuccess) return cuda_fail(e, what);
+  g_last_launch[0] = 0; g_last_launch[1] = 0; g_last_launch[2] = 0; g_last_launch[3] = kEngWide;
+  record_variant(kEngWide, 0, 0, false);
+  return 0;
+}
+
 static unsigned long long dp_timeout_ns() {
   unsigned long long ms = 20000ULL;   // a rank that is this late is gone (CNFOT_DP_TIMEOUT_MS overrides)
   if (const char* e = getenv("CNFOT_DP_TIMEOUT_MS")) {
@@ -860,11 +894,8 @@ static int mfc_step_impl(void* stream, const cnfot_flow_desc* flow, const cnfot_
   if (int rc = check_flow(flow, &lay)) return rc;
   if (use_wide(flow, lay)) {
     cnfot_workspace_release(workspace);   // the wide engine uses the memory as plain scratch: not clean afterwards
-    if (io.rng || io.stateful)
-      return fail(CNFOT_ERR_ARG, "the wide-conditioner engine takes explicit row arrays: fill them with cnfot_philox_rows "
-                                 "and call cnfot_mfc_step (+ cnfot_adam_update)");
-    return mfc_step_wide(stream, flow, lay, problem, weights, io.latent, io.latent_sub, io.src, io.tgt, io.t_batch_host, n_t,
-                         rows_B, rows_b, global_B, global_b, lambda, io.out, workspace, workspace_bytes, io.accumulate, io.peers);
+    return mfc_step_wide(stream, flow, lay, problem, weights, io, n_t, rows_B, rows_b, global_B, global_b, lambda, workspace,
+                         workspace_bytes);
   }
   if (int rc = check_fused(flow, lay)) return rc;
   if (!problem) return fail(CNFOT_ERR_ARG, "problem descriptor is NULL");
@@ -969,10 +1000,11 @@ static int mfc_step_impl(void* stream, const cnfot_flow_desc* flow, const cnfot_
   a.key = io.key;
   a.step = io.step;
   a.timeline = g_step_timeline;
-  a.salt_B = philox_salt(kDrawNormal, (uint64_t)global_B);
-  a.salt_Bc = philox_salt(kDrawCategorical, (uint64_t)global_B);
-  a.salt_b = philox_salt(kDrawNormal, (uint64_t)global_b);
-  a.salt_t = philox_salt(kDrawUniform, (uint64_t)n_t);
+  const StepSalts salts = step_salts(global_B, global_b, n_t);
+  a.salt_B = salts.B;
+  a.salt_Bc = salts.Bc;
+  a.salt_b = salts.b;
+  a.salt_t = salts.t;
   LaunchCfg cfg;
   if (int rc = configure(kernel, sp, (tiles * unit + kTile - 1) / kTile, &cfg, stash_cols)) return rc;
   record_variant(engine, stash_cols, group, engine == kEngMmaStream && group == 1 && latency);
@@ -1137,20 +1169,33 @@ int cnfot_mfc_step_rng(void* stream, const cnfot_flow_desc* flow, const cnfot_pr
 int64_t cnfot_train_state_bytes(const cnfot_flow_desc* flow) {
   FlowLayout lay;
   if (check_flow(flow, &lay)) return -1;
-  if (use_wide(flow, lay)) { fail(CNFOT_ERR_ARG, "no device-resident update for the wide-conditioner engine"); return -1; }
+  if (use_wide(flow, lay)) {
+    fail(CNFOT_ERR_ARG, "the wide-conditioner engine sizes its train state by the row counts: cnfot_train_state_bytes_rows");
+    return -1;
+  }
   return partial_bytes(lay);
+}
+
+int64_t cnfot_train_state_bytes_rows(const cnfot_flow_desc* flow, int64_t rows_B, int64_t rows_b) {
+  FlowLayout lay;
+  if (check_flow(flow, &lay)) return -1;
+  if (!use_wide(flow, lay)) return cnfot_train_state_bytes(flow);
+  if (rows_B < 0 || rows_b < 0) { fail(CNFOT_ERR_ARG, "bad row counts"); return -1; }
+  return wide_train_state_bytes(lay, rows_B, rows_b);
 }
 
 int cnfot_train_state_init(void* stream, const cnfot_flow_desc* flow, void* state, int64_t state_bytes, uint64_t key,
                            uint64_t step, uint32_t epoch) {
-  const int64_t need = cnfot_train_state_bytes(flow);
+  FlowLayout lay;
+  if (int rc = check_flow(flow, &lay)) return rc;
+  const bool wide = use_wide(flow, lay);
+  // wide flows: only the header is initialised here (the update checks the whole size against its row counts)
+  const int64_t need = wide ? kCounterBytes : cnfot_train_state_bytes(flow);
   if (need < 0) return CNFOT_ERR_ARG;
   if (!state) return fail(CNFOT_ERR_ARG, "NULL buffer");
   if (state_bytes < need) return fail(CNFOT_ERR_WORKSPACE, "train state too small: %lld < %lld", (long long)state_bytes, (long long)need);
-  FlowLayout lay;
-  check_flow(flow, &lay);
   cudaStream_t s = (cudaStream_t)stream;
-  cudaError_t e = cudaMemsetAsync(state, 0, (size_t)kCounterBytes + (size_t)kStepRows * lay.total * sizeof(float), s);
+  cudaError_t e = cudaMemsetAsync(state, 0, wide ? (size_t)kCounterBytes : (size_t)kCounterBytes + (size_t)kStepRows * lay.total * sizeof(float), s);
   if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync");
   const unsigned long long words[3] = {key, step, (unsigned long long)epoch};
   e = cudaMemcpyAsync((unsigned long long*)state + kStateWordOffset, words, sizeof(words), cudaMemcpyHostToDevice, s);

@@ -46,6 +46,18 @@ CNFOT_PHILOX_HD uint64_t splitmix64(uint64_t z) {
 // key modifier of a draw of `n` leading entries of kind `kind`
 CNFOT_PHILOX_HD uint64_t philox_salt(int kind, uint64_t n) { return splitmix64(splitmix64((uint64_t)kind) ^ n); }
 
+// The key modifiers of one train step's draws (both engines): normal (B, D) rows of the fit terms, categorical (B,)
+// mixture modes of the ot source, normal (b, D) rows of the kinetic terms, uniform (n_t,) times
+struct StepSalts { uint64_t B, Bc, b, t; };
+CNFOT_PHILOX_HD StepSalts step_salts(int64_t global_B, int64_t global_b, int n_t) {
+  StepSalts s;
+  s.B = philox_salt(kDrawNormal, (uint64_t)global_B);
+  s.Bc = philox_salt(kDrawCategorical, (uint64_t)global_B);
+  s.b = philox_salt(kDrawNormal, (uint64_t)global_b);
+  s.t = philox_salt(kDrawUniform, (uint64_t)n_t);
+  return s;
+}
+
 struct PhiloxWords { uint32_t w[4]; };
 
 CNFOT_PHILOX_HD uint32_t philox_mulhi(uint32_t a, uint32_t b) {
@@ -133,6 +145,36 @@ CNFOT_PHILOX_HD void philox_row(uint64_t key_n, uint64_t key_c, uint32_t step, i
       for (int j = 0; j < D; ++j) out[j] -= 3.0f;   // Gaussian -> Gaussian variant (applications.py:28-32, ot.py:72-80)
     }
   }
+}
+
+// Column c alone of philox_row's row (the same operations on the same words): for kernels that write one element
+// per thread
+CNFOT_PHILOX_HD float philox_entry(uint64_t key_n, uint64_t key_c, uint32_t step, int source, uint64_t row, int D, int c) {
+  const PhiloxWords p = philox_draw(key_n, step, row, (uint32_t)(c >> 2));
+  const int pair = (c >> 1) & 1;
+  float z0, z1;
+  philox_normal2(p.w[2 * pair], p.w[2 * pair + 1], z0, z1);
+  float v = (c & 1) ? z1 : z0;
+  if (source == kRowsOtSource) {
+    if (D == 2) {
+      const uint32_t idx = philox_draw(key_c, step, row, 0).w[0] >> 29;
+      float cx = 0.f, cy = 0.f;   // the modes of philox_row
+      switch (idx) {
+        case 0: cy = 5.0f; break;
+        case 1: cx = 5.0f; break;
+        case 2: cy = -5.0f; break;
+        case 3: cx = -5.0f; break;
+        case 4: cx = 3.0f; cy = 4.0f; break;
+        case 5: cx = 3.0f; cy = -4.0f; break;
+        case 6: cx = -3.0f; cy = -4.0f; break;
+        default: cx = -3.0f; cy = 4.0f; break;
+      }
+      v += c == 0 ? cx : cy;
+    } else {
+      v -= 3.0f;
+    }
+  }
+  return v;
 }
 
 }  // namespace cnfot

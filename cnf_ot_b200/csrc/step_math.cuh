@@ -400,4 +400,21 @@ CNFOT_HD T row_kinetic_value(const DimsT& dm, const SC& sc, T t, const T* latent
   return acc;
 }
 
+// ---- optax.adam (scale_by_adam + scale(-lr); cnf_ot/mfc/solvers.py:55,95-96) of the wide engine's device-resident update
+// The arithmetic of the fused tail (step_tail / adam_one in flow_kernels.cuh, which keep their own copy: routing the
+// fused kernels through these helpers changed their instruction schedule).  Bias corrections of update number `stepno`
+// (0-based): 1 - b^(stepno + 1) without the cancellation, -expm1((stepno + 1) log b); float32 is accurate to ~2e-7
+// relative here (optax itself evaluates 1 - b ** count in float32)
+CNFOT_HD void adam_bias(uint32_t stepno, float b1, float b2, float& c1, float& c2) {
+  const float n1 = (float)stepno + 1.f;
+  c1 = -expm1f(n1 * logf(b1));
+  c2 = -expm1f(n1 * logf(b2));
+}
+// one parameter: the old moments and parameter (m, v, w) in, the new ones out
+CNFOT_HD void adam_elem(float lr, float b1, float b2, float eps, float c1, float c2, float g, float& m, float& v, float& w) {
+  m = b1 * m + (1.f - b1) * g;
+  v = b2 * v + (1.f - b2) * g * g;
+  w = w - lr * (m / c1) / (sqrtf(v / c2) + eps);
+}
+
 }  // namespace cnfot

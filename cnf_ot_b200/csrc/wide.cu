@@ -113,19 +113,70 @@ wide_prep_kernel(const float* __restrict__ W, FlowLayout lay, WideDims wd, float
   }
 }
 
+// ---- where a pass's rows and time come from -------------------------------------------------------------------
+// Explicit: rows [r0, r0 + n) of an array and a time value.  Drawn: the rows of the step's Philox draw (philox.cuh, the
+// numbers the fused step kernel and cnfot_philox_rows / _times_host produce), global row row0 + r, and, with
+// t_index >= 0, the step's uniform time t_index plus `t` (the kinetic passes' -dt/2, +dt/2, 0).
+struct PassSrc {
+  const float* rows;   // (n x D) explicit rows, or NULL: drawn
+  float t;
+  int source;          // kRowsNormal / kRowsOtSource (drawn)
+  int t_index;         // drawn time index, or -1: `t` alone
+  uint64_t salt;       // key modifier of the normal draw: StepSalts::B or ::b
+  int64_t row0;
+};
+inline PassSrc explicit_src(const float* rows, float t) {
+  PassSrc p = {};
+  p.rows = rows;
+  p.t = t;
+  p.t_index = -1;
+  return p;
+}
+// key and step of the draws: by value, or read from the train state's words [key, step] (device-resident update)
+struct DrawKey {
+  uint64_t key;
+  uint32_t step;
+  const unsigned long long* state;
+  uint64_t salt_c, salt_t;   // categorical (ot source modes) and uniform (times) key modifiers
+  float horizon;
+};
+struct PassDraw {   // a DrawKey resolved inside a kernel
+  uint64_t key;
+  uint32_t step;
+};
+__device__ __forceinline__ PassDraw resolve(const DrawKey& dk) {
+  PassDraw d{dk.key, dk.step};
+  if (dk.state) {
+    d.key = __ldcg(dk.state);
+    d.step = (uint32_t)__ldcg(dk.state + 1);
+  }
+  return d;
+}
+__device__ __forceinline__ float pass_time(const PassSrc& ps, const DrawKey& dk, const PassDraw& d) {
+  return ps.t_index >= 0 ? philox_time(d.key ^ dk.salt_t, d.step, ps.t_index, dk.horizon) + ps.t : ps.t;
+}
+// column c < D of row r of the pass (explicit rows: ld_rows floats apart)
+__device__ __forceinline__ float pass_entry(const PassSrc& ps, const DrawKey& dk, const PassDraw& d, int64_t r, int ld_rows,
+                                            int D, int c) {
+  if (ps.rows) return ps.rows[r * ld_rows + c];
+  return philox_entry(d.key ^ ps.salt, d.key ^ dk.salt_c, d.step, ps.source, (uint64_t)(ps.row0 + r), D, c);
+}
+
 // ---- chunk state initialisation: S[0] = [rows | t | 0], S[1..L] = [0 | t | 0] ---------------------------
 __global__ void __launch_bounds__(kThreads)
-wide_init_kernel(const float* __restrict__ rows, int ld_rows, int64_t n, int D, int Kx, int L, int64_t state_stride, float t,
+wide_init_kernel(PassSrc ps, DrawKey dk, int ld_rows, int64_t n, int D, int Kx, int L, int64_t state_stride,
                  const float* __restrict__ cond, int64_t cond_stride, int shift_col, float shift, float* __restrict__ S) {
   const int64_t per = n * Kx;
   const int64_t total = per * (L + 1);
+  const PassDraw d = !ps.rows || ps.t_index >= 0 ? resolve(dk) : PassDraw{0, 0};
+  const float t = pass_time(ps, dk, d);
   for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
     const int s = (int)(e / per);
     const int64_t q = e - (int64_t)s * per;
     const int64_t r = q / Kx;
     const int c = (int)(q - r * Kx);
     float v = 0.f;
-    if (c < D) v = s == 0 ? rows[r * ld_rows + c] + (c == shift_col ? shift : 0.f) : 0.f;
+    if (c < D) v = s == 0 ? pass_entry(ps, dk, d, r, ld_rows, D, c) + (c == shift_col ? shift : 0.f) : 0.f;
     else if (c == D) v = cond ? cond[r * cond_stride] : t;
     S[(int64_t)s * state_stride + q] = v;
   }
@@ -786,14 +837,17 @@ wide_density_head_kernel(const float* __restrict__ Z, const float* __restrict__ 
 // ---- batched passes: several flow passes that start from the same rows share ONE chunk ---------------------------
 // (rows [j n, (j + 1) n) of the chunk = pass j).  Fewer, larger launches: a small-batch step is launch-bound.
 struct MultiSrc {
-  const float* src[3];
-  float t[3];
+  PassSrc src[3];
 };
 // state 0 = [src_j rows | t_j | 0] for j < reps, states 1..L = [0 | t_j | 0]
 __global__ void __launch_bounds__(kThreads)
-wide_init_multi_kernel(MultiSrc ms, int64_t n, int reps, int D, int Kx, int L, int64_t state_stride, float* __restrict__ S) {
+wide_init_multi_kernel(MultiSrc ms, DrawKey dk, int64_t n, int reps, int D, int Kx, int L, int64_t state_stride,
+                       float* __restrict__ S) {
   const int64_t per = n * reps * Kx;
   const int64_t total = per * (L + 1);
+  // every source of one chunk is drawn or none is (unused entries: zeroed)
+  const PassDraw d = !ms.src[0].rows ? resolve(dk) : PassDraw{0, 0};
+  const float tj[3] = {pass_time(ms.src[0], dk, d), pass_time(ms.src[1], dk, d), pass_time(ms.src[2], dk, d)};
   for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
     const int s = (int)(e / per);
     const int64_t q = e - (int64_t)s * per;
@@ -802,14 +856,15 @@ wide_init_multi_kernel(MultiSrc ms, int64_t n, int reps, int D, int Kx, int L, i
     const int j = (int)(row / n);
     const int64_t r = row - (int64_t)j * n;
     float v = 0.f;
-    if (c < D) v = s == 0 ? ms.src[j][r * D + c] : 0.f;
-    else if (c == D) v = ms.t[j];
+    if (c < D) v = s == 0 ? pass_entry(ms.src[j], dk, d, r, D, D, c) : 0.f;
+    else if (c == D) v = j == 0 ? tj[0] : (j == 1 ? tj[1] : tj[2]);
     S[(int64_t)s * state_stride + q] = v;
   }
 }
-// the 2 D shifted copies of the rows R3 (n x Kx): copy j = 2 i + side is R3 + (side ? -shift : +shift) e_i, all at time t
+// the 2 D shifted copies of the rows R3 (n x Kx): copy j = 2 i + side is R3 + (side ? -shift : +shift) e_i, all at the
+// time of R3 (its column D)
 __global__ void __launch_bounds__(kThreads)
-wide_init_shift_kernel(const float* __restrict__ R3, int64_t n, int D, int Kx, int L, int64_t state_stride, float t, float shift,
+wide_init_shift_kernel(const float* __restrict__ R3, int64_t n, int D, int Kx, int L, int64_t state_stride, float shift,
                        float* __restrict__ S) {
   const int64_t per = n * 2 * D * Kx;
   const int64_t total = per * (L + 1);
@@ -822,7 +877,7 @@ wide_init_shift_kernel(const float* __restrict__ R3, int64_t n, int D, int Kx, i
     const int64_t r = row - (int64_t)j * n;
     float v = 0.f;
     if (c < D) v = s == 0 ? R3[r * Kx + c] + (c == (j >> 1) ? ((j & 1) ? -shift : shift) : 0.f) : 0.f;
-    else if (c == D) v = t;
+    else if (c == D) v = R3[r * Kx + D];
     S[(int64_t)s * state_stride + q] = v;
   }
 }
@@ -896,6 +951,35 @@ __global__ void wide_finalize_kernel(const double* __restrict__ slots, float* __
     out_slots[3] = (float)slots[kSlotPotential];
     out_slots[4] = (float)slots[kSlotKinetic];
     out_slots[5] = out_slots[6] = out_slots[7] = 0.f;
+  }
+}
+
+// ---- the device-resident update's tail: optax.adam on the step's gradient (adam_elem, shared with the fused tail) ----
+// out = [gradient (total) | loss slots]; update number state[1]; a NaN gradient entry leaves its parameter alone
+__global__ void __launch_bounds__(kThreads)
+wide_adam_kernel(const float* __restrict__ out, int64_t total, const unsigned long long* __restrict__ state, float lr, float b1,
+                 float b2, float eps, float* __restrict__ W, float* __restrict__ m, float* __restrict__ v,
+                 float* __restrict__ loss_hist, int64_t loss_hist_len) {
+  const uint32_t stepno = (uint32_t)__ldcg(state + 1);
+  float c1, c2;
+  adam_bias(stepno, b1, b2, c1, c2);
+  const int64_t i0 = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i0 == 0 && loss_hist && (int64_t)stepno < loss_hist_len) loss_hist[stepno] = out[total];
+  for (int64_t i = i0; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const float g = out[i];
+    if (g != g) continue;
+    float mi = m[i], vi = v[i], wi = W[i];
+    adam_elem(lr, b1, b2, eps, c1, c2, g, mi, vi, wi);
+    m[i] = mi;
+    v[i] = vi;
+    W[i] = wi;
+  }
+}
+// after every block of wide_adam_kernel has read it: the next update's number (and epoch, as the fused tail keeps it)
+__global__ void wide_advance_kernel(unsigned long long* __restrict__ state) {
+  if (threadIdx.x == 0) {
+    state[1] += 1ULL;
+    state[2] += 1ULL;
   }
 }
 
@@ -991,6 +1075,7 @@ struct WideEngine {
   float* stashA;          // n_mlp x R x H: last hidden activations of pass 0, kept for its backward sweep (or NULL)
   float* stashT;          // n_mlp x R x Pp: raw spline parameters of pass 0
   double* slots;
+  DrawKey dk = {};        // the step's draws (passes whose rows are not explicit)
   cudaError_t err = cudaSuccess;
   const char* what = "";
 
@@ -1140,16 +1225,19 @@ struct WideEngine {
     check_launch("wide_spline_vjp_kernel launch");
   }
 
-  // state 0 of pass p = [rows (+ shift on one coordinate) | t | 0]; ld_rows = row stride of `rows` (0: dense, D)
-  void init_states(int p, const float* rows, int64_t n, float t, const float* cond = nullptr, int64_t cond_stride = 0,
+  // state 0 of pass p = [rows (+ shift on one coordinate) | t | 0]; ld_rows = row stride of explicit rows (0: dense, D)
+  void init_states(int p, const PassSrc& ps, int64_t n, const float* cond = nullptr, int64_t cond_stride = 0,
                    int ld_rows = 0, int shift_col = -1, float shift = 0.f) {
     if (!ok()) return;
     int64_t total = n * wd.Kx * (wd.L + 1);
     int64_t b = (total + kThreads - 1) / kThreads;
     if (b > 148 * 16) b = 148 * 16;
-    wide_init_kernel<<<(unsigned)b, kThreads, 0, s>>>(rows, ld_rows ? ld_rows : wd.D, n, wd.D, wd.Kx, wd.L, state_stride(), t, cond,
-                                                      cond_stride, shift_col, shift, S[p]);
+    wide_init_kernel<<<(unsigned)b, kThreads, 0, s>>>(ps, dk, ld_rows ? ld_rows : wd.D, n, wd.D, wd.Kx, wd.L, state_stride(),
+                                                      cond, cond_stride, shift_col, shift, S[p]);
     check_launch("wide_init_kernel launch");
+  }
+  void init_states(int p, const float* rows, int64_t n, float t, const float* cond = nullptr, int64_t cond_stride = 0) {
+    init_states(p, explicit_src(rows, t), n, cond, cond_stride);
   }
 
   static unsigned grid_for(int64_t count) {
@@ -1159,14 +1247,14 @@ struct WideEngine {
   // pass p = `reps` passes over the same n rows (sources / times per pass in ms), stacked in one chunk
   void init_multi(int p, const MultiSrc& ms, int64_t n, int reps) {
     if (!ok()) return;
-    wide_init_multi_kernel<<<grid_for(n * reps * wd.Kx * (wd.L + 1)), kThreads, 0, s>>>(ms, n, reps, wd.D, wd.Kx, wd.L,
+    wide_init_multi_kernel<<<grid_for(n * reps * wd.Kx * (wd.L + 1)), kThreads, 0, s>>>(ms, dk, n, reps, wd.D, wd.Kx, wd.L,
                                                                                         state_stride(), S[p]);
     check_launch("wide_init_multi_kernel launch");
   }
-  void init_shift(int p, const float* R3, int64_t n, float t, float shift) {
+  void init_shift(int p, const float* R3, int64_t n, float shift) {
     if (!ok()) return;
     wide_init_shift_kernel<<<grid_for(n * 2 * wd.D * wd.Kx * (wd.L + 1)), kThreads, 0, s>>>(R3, n, wd.D, wd.Kx, wd.L,
-                                                                                            state_stride(), t, shift, S[p]);
+                                                                                            state_stride(), shift, S[p]);
     check_launch("wide_init_shift_kernel launch");
   }
   void fill(float* p, int64_t count, float v) {
@@ -1299,18 +1387,24 @@ void launch_prep(WideEngine& e, bool with_T) {
   e.check_launch("wide_prep_kernel launch");
 }
 
-// kinetic terms of one chunk of the b-row sub-batch at time t (row_kinetic of step_math.cuh)
+// the same rows at time t + dt (t - dt / 2 == t + (-dt / 2) exactly: the times of row_kinetic in step_math.cuh)
+inline PassSrc at_time(PassSrc ps, float dt) {
+  ps.t = ps.t + dt;
+  return ps;
+}
+
+// kinetic terms of one chunk of the b-row sub-batch: `rt` = its rows at time t (row_kinetic of step_math.cuh)
 template <int K>
-void kinetic_chunk(WideEngine& e, const StepConsts<float>& pc, const float* rows, int64_t n, float t) {
+void kinetic_chunk(WideEngine& e, const StepConsts<float>& pc, const PassSrc& rt, int64_t n) {
   const int D = e.wd.D, Kx = e.wd.Kx, L = e.wd.L;
   const bool with_score = pc.type != kOT;
   const bool obstacle = pc.potential == kPotObstacle && !with_score;
-  e.init_states(0, rows, n, t - pc.dt / 2.f);
-  e.init_states(1, rows, n, t + pc.dt / 2.f);
+  e.init_states(0, at_time(rt, -pc.dt / 2.f), n);
+  e.init_states(1, at_time(rt, pc.dt / 2.f), n);
   e.flow_pass<K>(0, 0, n);
   e.flow_pass<K>(0, 1, n);
   if (obstacle || with_score) {
-    e.init_states(2, rows, n, t);
+    e.init_states(2, rt, n);
     e.flow_pass<K>(0, 2, n);
   }
   if (!e.ok()) return;
@@ -1328,9 +1422,11 @@ void kinetic_chunk(WideEngine& e, const StepConsts<float>& pc, const float* rows
     int64_t ab = (n * Kx + kThreads - 1) / kThreads;
     if (ab > 148 * 16) ab = 148 * 16;
     for (int i = 0; i < D && e.ok(); ++i) {
-      // the two log-prob passes of coordinate i start from r3 -+ e_i dx/2: forward both, then back-propagate both
-      e.init_states(3, e.state(2, L), n, t, nullptr, 0, Kx, i, pc.dx / 2.f);
-      e.init_states(4, e.state(2, L), n, t, nullptr, 0, Kx, i, -pc.dx / 2.f);
+      // the two log-prob passes of coordinate i start from r3 -+ e_i dx/2 at the time of r3: forward both, then
+      // back-propagate both
+      const float* r3 = e.state(2, L);
+      e.init_states(3, explicit_src(r3, 0.f), n, r3 + D, Kx, Kx, i, pc.dx / 2.f);
+      e.init_states(4, explicit_src(r3, 0.f), n, r3 + D, Kx, Kx, i, -pc.dx / 2.f);
       e.flow_pass<K>(1, 3, n);
       e.flow_pass<K>(1, 4, n);
       if (!e.ok()) return;
@@ -1364,14 +1460,13 @@ bool batching_enabled() {
 // direction pass of 2-3 n rows and the 2 D shifted log-prob passes of the score are ONE pass of 2 D n rows.
 // Requires 3 n <= R and (score) 2 D n <= R.
 template <int K>
-void kinetic_chunk_batched(WideEngine& e, const StepConsts<float>& pc, const float* rows, int64_t n, float t) {
+void kinetic_chunk_batched(WideEngine& e, const StepConsts<float>& pc, const PassSrc& rt, int64_t n) {
   const int D = e.wd.D, Kx = e.wd.Kx, L = e.wd.L;
   const bool with_score = pc.type != kOT;
   const bool obstacle = pc.potential == kPotObstacle && !with_score;
   const int reps = (obstacle || with_score) ? 3 : 2;
   MultiSrc ms;
-  for (int j = 0; j < 3; ++j) ms.src[j] = rows;
-  ms.t[0] = t - pc.dt / 2.f; ms.t[1] = t + pc.dt / 2.f; ms.t[2] = t;
+  ms.src[0] = at_time(rt, -pc.dt / 2.f); ms.src[1] = at_time(rt, pc.dt / 2.f); ms.src[2] = rt;
   e.init_multi(0, ms, n, reps);
   e.flow_pass<K>(0, 0, n * reps);
   if (!e.ok()) return;
@@ -1384,7 +1479,7 @@ void kinetic_chunk_batched(WideEngine& e, const StepConsts<float>& pc, const flo
         e.slots + kSlotKinetic, e.slots + kSlotPotential);
     e.check_launch("wide_kinetic_head_kernel launch");
   } else {
-    e.init_shift(1, r1 + 2 * blk, n, t, pc.dx / 2.f);
+    e.init_shift(1, r1 + 2 * blk, n, pc.dx / 2.f);
     e.flow_pass<K>(1, 1, n * 2 * D);
     if (!e.ok()) return;
     wide_score_head_all_kernel<<<WideEngine::blocks_for(n), kThreads, 0, e.s>>>(
@@ -1403,9 +1498,27 @@ void kinetic_chunk_batched(WideEngine& e, const StepConsts<float>& pc, const flo
   e.flow_bwd<K>(0, 0, n * reps, 0.f, nullptr);
 }
 
+// the step's row sets: the caller's arrays and host times, or (draws != NULL) the Philox draws of the step
+struct StepRows {
+  const float *latent, *latent_sub, *src, *tgt, *t_batch_host;
+  const WideDraws* draws;
+  int D;
+  // rows [r0, r0 + n) of a row set of the B-row terms (sub = false) or of the b-row kinetic terms (sub = true) at time t,
+  // plus, with t_index >= 0, the step's time t_index
+  PassSrc at(const float* rows, int source, bool sub, int64_t r0, float t, int t_index = -1) const {
+    if (!draws) return explicit_src(rows + r0 * D, t_index >= 0 ? t_batch_host[t_index] + t : t);
+    PassSrc p = {};
+    p.t = t;
+    p.source = source;
+    p.t_index = t_index;
+    p.salt = sub ? draws->salts.b : draws->salts.B;
+    p.row0 = (sub ? draws->row0_b : draws->row0_B) + r0;
+    return p;
+  }
+};
+
 template <int K>
-void run_step(WideEngine& e, const StepConsts<float>& pc, const float* latent, const float* latent_sub, const float* src,
-              const float* tgt, const float* t_batch_host, int n_t, int64_t rows_B, int64_t rows_b) {
+void run_step(WideEngine& e, const StepConsts<float>& pc, const StepRows& in, int n_t, int64_t rows_B, int64_t rows_b) {
   const int D = e.wd.D, Kx = e.wd.Kx, L = e.wd.L;
   const bool batch = batching_enabled();
   // kinetic terms: the b-row sub-batch at every sampled time
@@ -1417,8 +1530,9 @@ void run_step(WideEngine& e, const StepConsts<float>& pc, const float* latent, c
     if (!stacked) cap = e.R;
     for (int64_t r0 = 0; r0 < rows_b && e.ok(); r0 += cap) {
       const int64_t n = rows_b - r0 < cap ? rows_b - r0 : cap;
-      if (stacked) kinetic_chunk_batched<K>(e, pc, latent_sub + r0 * D, n, t_batch_host[it]);
-      else kinetic_chunk<K>(e, pc, latent_sub + r0 * D, n, t_batch_host[it]);
+      const PassSrc rt = in.at(in.latent_sub, kRowsNormal, true, r0, 0.f, it);
+      if (stacked) kinetic_chunk_batched<K>(e, pc, rt, n);
+      else kinetic_chunk<K>(e, pc, rt, n);
     }
   }
   const int64_t half = e.R / 2;
@@ -1429,8 +1543,8 @@ void run_step(WideEngine& e, const StepConsts<float>& pc, const float* latent, c
       for (int64_t r0 = 0; r0 < rows_B && e.ok(); r0 += half) {
         const int64_t n = rows_B - r0 < half ? rows_B - r0 : half;
         MultiSrc ms;
-        ms.src[0] = src + r0 * D; ms.src[1] = tgt + r0 * D; ms.src[2] = nullptr;
-        ms.t[0] = 0.f; ms.t[1] = pc.horizon; ms.t[2] = 0.f;
+        ms.src[0] = in.at(in.src, kRowsOtSource, false, r0, 0.f);
+        ms.src[1] = ms.src[2] = in.at(in.tgt, kRowsNormal, false, r0, pc.horizon);
         e.init_multi(0, ms, n, 2);
         e.flow_pass<K>(1, 0, 2 * n, true);
         if (!e.ok()) break;
@@ -1445,12 +1559,11 @@ void run_step(WideEngine& e, const StepConsts<float>& pc, const float* latent, c
       return;
     }
     for (int side = 0; side < 2 && e.ok(); ++side) {
-      const float* data = side == 0 ? src : tgt;
       const float t = side == 0 ? 0.f : pc.horizon;
       double* slot = e.slots + (side == 0 ? kSlotFit0 : kSlotFitT);
       for (int64_t r0 = 0; r0 < rows_B && e.ok(); r0 += e.R) {
         const int64_t n = rows_B - r0 < e.R ? rows_B - r0 : e.R;
-        e.init_states(0, data + r0 * D, n, t);
+        e.init_states(0, side == 0 ? in.at(in.src, kRowsOtSource, false, r0, t) : in.at(in.tgt, kRowsNormal, false, r0, t), n);
         e.flow_pass<K>(1, 0, n, true);
         if (!e.ok()) break;
         wide_nll_head_kernel<<<WideEngine::blocks_for(n), kThreads, 0, e.s>>>(e.state(0, L), e.LD[0], n, D, Kx, pc.w_fit,
@@ -1469,14 +1582,14 @@ void run_step(WideEngine& e, const StepConsts<float>& pc, const float* latent, c
     for (int64_t r0 = 0; r0 < rows_B && e.ok(); r0 += half) {
       const int64_t n = rows_B - r0 < half ? rows_B - r0 : half;
       MultiSrc ms;
-      ms.src[0] = latent + r0 * D; ms.src[1] = latent + r0 * D; ms.src[2] = nullptr;
-      ms.t[0] = 0.f; ms.t[1] = pc.horizon; ms.t[2] = 0.f;
+      ms.src[0] = in.at(in.latent, kRowsNormal, false, r0, 0.f);
+      ms.src[1] = ms.src[2] = in.at(in.latent, kRowsNormal, false, r0, pc.horizon);
       e.init_multi(0, ms, n, 2);
       e.flow_pass<K>(0, 0, 2 * n, true);
       if (!e.ok()) break;
       for (int seg = 0; seg < 2; ++seg) {
         wide_sample_head_kernel<<<WideEngine::blocks_for(n), kThreads, 0, e.s>>>(
-            e.state(0, 0) + seg * n * Kx, e.state(0, L) + seg * n * Kx, e.LD[0] + seg * n, n, D, Kx, ms.t[seg], seg == 0,
+            e.state(0, 0) + seg * n * Kx, e.state(0, L) + seg * n * Kx, e.LD[0] + seg * n, n, D, Kx, seg == 0 ? 0.f : pc.horizon, seg == 0,
             seg == 1, pc, e.G[0] + seg * n * Kx, e.slots + kSlotFit0, e.slots + kSlotPotential);
         e.check_launch("wide_sample_head_kernel launch");
       }
@@ -1491,7 +1604,7 @@ void run_step(WideEngine& e, const StepConsts<float>& pc, const float* latent, c
     const float t = seg == 0 ? 0.f : pc.horizon;
     for (int64_t r0 = 0; r0 < rows_B && e.ok(); r0 += e.R) {
       const int64_t n = rows_B - r0 < e.R ? rows_B - r0 : e.R;
-      e.init_states(0, latent + r0 * D, n, t);
+      e.init_states(0, in.at(in.latent, kRowsNormal, false, r0, t), n);
       e.flow_pass<K>(0, 0, n, true);
       if (!e.ok()) break;
       wide_sample_head_kernel<<<WideEngine::blocks_for(n), kThreads, 0, e.s>>>(
@@ -1526,18 +1639,33 @@ int64_t wide_flow_workspace_bytes(const FlowLayout& lay, int64_t rows, bool with
 
 cudaError_t wide_mfc_step(cudaStream_t s, const FlowLayout& lay, const SplineConsts<float>& sc, const StepConsts<float>& pc,
                           const float* weights, const float* latent, const float* latent_sub, const float* src,
-                          const float* tgt, const float* t_batch_host, int n_t, int64_t rows_B, int64_t rows_b, float* out,
-                          void* workspace, const char** what) {
+                          const float* tgt, const float* t_batch_host, const WideDraws* draws, int n_t, int64_t rows_B,
+                          int64_t rows_b, float* out, const WideAdam* adam, void* workspace, const char** what) {
   WideEngine e;
   e.s = s; e.sc = sc; e.W = weights; e.grad = out;
   carve(workspace, lay, rows_B > rows_b ? rows_B : rows_b, true, kMaxPass, &e);
+  if (draws) {
+    e.dk.key = draws->key; e.dk.step = draws->step; e.dk.state = draws->state;
+    e.dk.salt_c = draws->salts.Bc; e.dk.salt_t = draws->salts.t; e.dk.horizon = pc.horizon;
+  }
   e.check(cudaMemsetAsync(out, 0, ((size_t)lay.total + kNumSlots) * sizeof(float), s), "cudaMemsetAsync");
   e.check(cudaMemsetAsync(e.slots, 0, kNumSlots * sizeof(double), s), "cudaMemsetAsync");
   launch_prep(e, true);
-  run_step<5>(e, pc, latent, latent_sub, src, tgt, t_batch_host, n_t, rows_B, rows_b);
+  StepRows in = {latent, latent_sub, src, tgt, t_batch_host, draws, lay.D};
+  run_step<5>(e, pc, in, n_t, rows_B, rows_b);
   if (e.ok()) {
     wide_finalize_kernel<<<1, 32, 0, s>>>(e.slots, out + lay.total);
     e.check_launch("wide_finalize_kernel launch");
+  }
+  if (adam && e.ok()) {
+    wide_adam_kernel<<<WideEngine::grid_for(lay.total), kThreads, 0, s>>>(out, lay.total, adam->state, adam->lr, adam->b1,
+                                                                          adam->b2, adam->eps, adam->weights, adam->m,
+                                                                          adam->v, adam->loss_hist, adam->loss_hist_len);
+    e.check_launch("wide_adam_kernel launch");
+    if (e.ok()) {
+      wide_advance_kernel<<<1, 32, 0, s>>>(adam->state);
+      e.check_launch("wide_advance_kernel launch");
+    }
   }
   if (what) *what = e.what;
   return e.err;
@@ -1634,8 +1762,8 @@ cudaError_t wide_kinetic_energy(cudaStream_t s, const FlowLayout& lay, const Spl
         e.init_states(2, rows, n, t);
         e.flow_pass<5>(0, 2, n);
         for (int i = 0; i < D && e.ok(); ++i) {
-          e.init_states(3, e.state(2, L), n, t, nullptr, 0, Kx, i, dx / 2.f);
-          e.init_states(4, e.state(2, L), n, t, nullptr, 0, Kx, i, -dx / 2.f);
+          e.init_states(3, explicit_src(e.state(2, L), t), n, nullptr, 0, Kx, i, dx / 2.f);
+          e.init_states(4, explicit_src(e.state(2, L), t), n, nullptr, 0, Kx, i, -dx / 2.f);
           e.flow_pass<5>(1, 3, n);
           e.flow_pass<5>(1, 4, n);
           if (!e.ok()) break;

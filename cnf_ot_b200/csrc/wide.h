@@ -6,6 +6,7 @@
 #include <stdint.h>
 
 #include "flow_math.cuh"
+#include "philox.cuh"
 #include "step_math.cuh"
 
 namespace cnfot {
@@ -15,11 +16,34 @@ bool wide_supported(const FlowLayout& lay, const char** why);
 int64_t wide_step_workspace_bytes(const FlowLayout& lay, int64_t rows_B, int64_t rows_b);
 int64_t wide_flow_workspace_bytes(const FlowLayout& lay, int64_t rows, bool with_grad);
 
-// value_and_grad of ot_loss_fn / rwpo_loss_fn / fp_loss_fn on this shard: out = [gradient (blob) | 8 loss slots], overwritten
+// The step's draws made on chip, the numbers of the fused step kernel (philox.cuh): key and step by value, or, with
+// `state` != NULL, read by the kernels from the train state's words [key, step] (a captured launch then draws the rows of
+// whichever update it runs as); salts = step_salts(global_B, global_b, n_t); row0_*: global index of the shard's first row
+struct WideDraws {
+  uint64_t key;
+  uint32_t step;
+  const unsigned long long* state;
+  StepSalts salts;
+  int64_t row0_B, row0_b;
+};
+// The device-resident update's tail: optax.adam with the step's gradient on weights / m / v in place, for update number
+// state[1]; loss_hist[state[1]] = total loss when state[1] < loss_hist_len; then state[1] and the epoch state[2] advance
+struct WideAdam {
+  unsigned long long* state;
+  float* weights;
+  float* m;
+  float* v;
+  float lr, b1, b2, eps;
+  float* loss_hist;
+  int64_t loss_hist_len;
+};
+
+// value_and_grad of ot_loss_fn / rwpo_loss_fn / fp_loss_fn on this shard: out = [gradient (blob) | 8 loss slots], overwritten.
+// Rows and times: the explicit arrays, or (draws != NULL) drawn on chip; adam != NULL: the update's tail follows
 cudaError_t wide_mfc_step(cudaStream_t s, const FlowLayout& lay, const SplineConsts<float>& sc, const StepConsts<float>& pc,
                           const float* weights, const float* latent, const float* latent_sub, const float* src,
-                          const float* tgt, const float* t_batch_host, int n_t, int64_t rows_B, int64_t rows_b, float* out,
-                          void* workspace, const char** what);
+                          const float* tgt, const float* t_batch_host, const WideDraws* draws, int n_t, int64_t rows_B,
+                          int64_t rows_b, float* out, const WideAdam* adam, void* workspace, const char** what);
 // flow.bijector.forward / inverse (dir 0 / 1) with log-det (or the density with add_base)
 cudaError_t wide_flow_eval(cudaStream_t s, const FlowLayout& lay, const SplineConsts<float>& sc, const float* weights,
                            int dir, const float* in, const float* cond, int64_t cond_stride, int64_t rows, float* out,

@@ -387,14 +387,19 @@ def fused_update_supported(shape: FlowShape) -> bool:
 
 
 class TrainState:
-  """Device-resident state of the fused update (cnfot_mfc_update): key, step count, all-reduce epoch and the step
-  kernel's self-cleaning reduction buffers, plus the optax.adam moments (solvers.py:55-56)."""
+  """Device-resident state of the update (cnfot_mfc_update): key, step count, all-reduce epoch and the step
+  kernel's self-cleaning reduction buffers, plus the optax.adam moments (solvers.py:55-56).
 
-  def __init__(self, shape: FlowShape, params_blob: torch.Tensor, key: int, step: int = 0, peers=None):
+  rows_B / rows_b: this shard's row counts of the updates the state will serve.  Flows on the wide-conditioner engine
+  need them (their state also holds the step's gradient and workspace, cnfot_train_state_bytes_rows); the fused
+  kernels' state does not depend on them."""
+
+  def __init__(self, shape: FlowShape, params_blob: torch.Tensor, key: int, step: int = 0, peers=None,
+               rows_B: int = 0, rows_b: int = 0):
     lib = _lib.load()
     self.shape, self.device = shape, params_blob.device
     self.desc = _lib.flow_desc(shape)
-    n = lib.cnfot_train_state_bytes(self.desc)
+    n = lib.cnfot_train_state_bytes_rows(self.desc, int(rows_B), int(rows_b))
     if n < 0:
       _lib.check(1)
     self.buf = torch.empty(n, dtype=torch.uint8, device=self.device)
@@ -425,8 +430,10 @@ class TrainState:
 def mfc_update(shape: FlowShape, problem: _lib.ProblemDesc, state: TrainState, weights: torch.Tensor, n_t: int, lam: float,
                global_B: int, global_b: int, lr: float, rows_B=None, rows_b=None, out: Optional[torch.Tensor] = None,
                loss_hist: Optional[torch.Tensor] = None, b1=0.9, b2=0.999, eps=1e-8) -> None:
-  """One `update` (solvers.py:90-97): value_and_grad on on-chip draws + all-reduce + Adam in ONE kernel launch.
-  Nothing host-side changes between calls, so a run of calls can be captured in a CUDA graph and replayed."""
+  """One `update` (solvers.py:90-97): value_and_grad on on-chip draws + all-reduce + Adam in ONE kernel launch
+  (wide-conditioner flows: a fixed sequence of launches, no all-reduce; the state must be sized for these rows).
+  Nothing host-side changes between calls, so a run of calls can be captured in a CUDA graph and replayed (after one
+  call outside the capture)."""
   lib = _lib.load()
   weights = _dev(weights, "weights")
   rB = slice(0, global_B) if rows_B is None else rows_B

@@ -81,8 +81,11 @@ def main(config_dict: Dict, progress: bool = False, graph_steps: int = None):
   Flows the fused step kernel covers train DEVICE-RESIDENT: one kernel launch per `update` (on-chip draws,
   value_and_grad, the data-parallel all-reduce, Adam: `cnfot_mfc_update`), `graph_steps` updates per CUDA graph
   (default: eval_frequency, at most 100), the loss history written by the kernel -- the host only replays graphs.
-  The draws of update k are those of (train key, step k).  Wide-conditioner flows take the update() loop of
-  `make_update` (one key per step, split from the run's key as in solvers.py:104)."""
+  The draws of update k are those of (train key, step k).  Wide-conditioner flows train the same way on one GPU
+  (their update is a fixed sequence of launches, captured the same way), so a single-GPU wide run also draws the
+  numbers of (train key, step k) -- before, it drew them from one key per step split from the run's key; with
+  several GPUs they take the update() loop of `make_update` (that per-step key, as in solvers.py:104, and an NCCL
+  all-reduce of the gradient)."""
   config = config_dict
   rng = random.PRNGKey(config["general"]["seed"])
   tr = config["train"]
@@ -115,14 +118,15 @@ def main(config_dict: Dict, progress: bool = False, graph_steps: int = None):
         print(desc, flush=True)
     return rng
 
-  if ops.fused_update_supported(model.shape) and params.blob.is_cuda:
+  if params.blob.is_cuda and (ops.fused_update_supported(model.shape) or world == 1):
     sc = applications._step_config(loss_fn)
     shape, problem, n_t = model.shape, sc["problem"], config["general"]["t_batch_size"]
     B, b = batch_size, batch_size // 32
     rs, ss = applications._dist.shard(B, rank, world), applications._dist.shard(b, rank, world)
     train_key, rng = random.split(rng)
     key = int(resume["rng/train_key"]) if resume and "rng/train_key" in resume else train_key.value
-    state = ops.TrainState(shape, params.blob, key, step=step0, peers=applications.peer_exchange(shape, model.device))
+    state = ops.TrainState(shape, params.blob, key, step=step0, peers=applications.peer_exchange(shape, model.device),
+                           rows_B=rs.stop - rs.start, rows_b=ss.stop - ss.start)
     if resume and "opt/mu" in resume:
       state.mu.copy_(resume["opt/mu"].to(state.mu.device))
       state.nu.copy_(resume["opt/nu"].to(state.nu.device))

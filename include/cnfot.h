@@ -266,8 +266,10 @@ CNFOT_API int cnfot_mfc_step_dp(void* stream, const cnfot_flow_desc* flow, const
  *                            sub-batch latent = NORMAL (global_b, dim), times = n_t uniforms; this rank's shard is
  *                            rows [row0_B, row0_B + rows_B) of the B-row terms and [row0_b, row0_b + rows_b) of
  *                            the b-row terms
+ *                            (both engines; the wide-conditioner engine draws straight into its chunk states and
+ *                            refuses `peers`: its workspace is cnfot_mfc_step_workspace_bytes())
  *   cnfot_mfc_step_rng_host  the same with HOST weights in and HOST [gradient | loss] out (transfers inside,
- *                            synchronises): the key is the only other input */
+ *                            synchronises): the key is the only other input (fused per-row kernels only) */
 enum { CNFOT_ROWS_NORMAL = 1,     /* N(0, I) rows: latent draws and the target of kl_loss_fn (applications.py:73-82) */
        CNFOT_ROWS_OT_SOURCE = 3   /* kl_loss_fn source: z + 8-mode mixture centre (dim 2, applications.py:34-71), z - 3
                                      otherwise; z = the NORMAL draw of the same shape (the reference reuses the key) */ };
@@ -292,9 +294,17 @@ CNFOT_API int cnfot_mfc_step_rng_host(void* stream, const cnfot_flow_desc* flow,
  * cnfot_train_state_bytes()) carries the key, the step count (starts at `step`, +1 per call: it selects the
  * draws, Adam's bias correction and the slot of loss_hist) and the all-reduce epoch, plus the kernel's
  * self-cleaning reduction buffers.  out (may be NULL): [gradient | loss slots] of the step; loss_hist (may be
- * NULL): loss_hist[step] = total loss when step < loss_hist_len.  weights, adam_m, adam_v are updated in place. */
+ * NULL): loss_hist[step] = total loss when step < loss_hist_len.  weights, adam_m, adam_v are updated in place.
+ * Flows on the wide-conditioner engine take the same calls: the update is then a sequence of stream-ordered launches
+ * (draws made by the chunk-state initialisation, the engine's step, an Adam kernel, a one-thread step advance) with no
+ * host synchronisation and no host-memory read, so it is captured like the fused one -- provided one update has run
+ * on the device OUTSIDE a capture first (it sets the kernels' shared-memory limits, which a capture must not be the
+ * first to do).  Their train state holds the step's gradient and workspace as well, so its size depends on the row
+ * counts: cnfot_train_state_bytes_rows(flow, rows_B, rows_b) (this shard's rows; equal to cnfot_train_state_bytes() for
+ * the fused kernels, which returns -1 for wide flows); no `peers` (all-reduce the gradient of cnfot_mfc_step with NCCL). */
 typedef struct cnfot_adam_desc { float lr, b1, b2, eps; } cnfot_adam_desc;   /* optax.adam defaults: b1 .9 b2 .999 eps 1e-8 */
 CNFOT_API int64_t cnfot_train_state_bytes(const cnfot_flow_desc* flow);
+CNFOT_API int64_t cnfot_train_state_bytes_rows(const cnfot_flow_desc* flow, int64_t rows_B, int64_t rows_b);
 CNFOT_API int cnfot_train_state_init(void* stream, const cnfot_flow_desc* flow, void* state, int64_t state_bytes,
                            uint64_t key, uint64_t step, uint32_t epoch);
 CNFOT_API int cnfot_mfc_update(void* stream, const cnfot_flow_desc* flow, const cnfot_problem_desc* problem,
