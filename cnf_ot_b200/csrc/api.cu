@@ -97,7 +97,12 @@ static int check_fused(const cnfot_flow_desc* f, const FlowLayout& lay) {
   if (!reference_spline_consts(f))
     return fail(CNFOT_ERR_ARG, "the fused flow kernels are compiled for the reference's spline constants (range -10..10, "
                                "min_bin_size = min_knot_slope = 1e-4; cnf_ot/models/flows.py:124-132)");
-  if (f->dim > kMaxDim) return fail(CNFOT_ERR_ARG, "fused kernels support dim <= %d (got %d)", kMaxDim, f->dim);
+  if (f->dim > kMaxDim) {
+    const char* why = nullptr;   // rows this wide are the wide engine's: say why it refused
+    if (!wide_supported(lay, &why))
+      return fail(CNFOT_ERR_ARG, "fused kernels support dim <= %d and %s (got %d)", kMaxDim, why, f->dim);
+    return fail(CNFOT_ERR_ARG, "fused kernels support dim <= %d (got %d)", kMaxDim, f->dim);
+  }
   if ((f->num_layers + 1) * f->dim > kMaxStateFloats)
     return fail(CNFOT_ERR_ARG, "fused kernels need (num_layers+1)*dim <= %d (got %d)", kMaxStateFloats,
                 (f->num_layers + 1) * f->dim);
@@ -1130,18 +1135,34 @@ philox_rows_kernel(unsigned long long key_n, unsigned long long key_c, uint32_t 
   }
 }
 
+// rows wider than kMaxDim: one element per thread (philox_entry: philox_row's numbers, no row-sized array)
+__global__ void __launch_bounds__(256)
+philox_entries_kernel(unsigned long long key_n, unsigned long long key_c, uint32_t step, int source, int64_t row0,
+                      int64_t rows, int dim, float* __restrict__ out) {
+  const int64_t total = rows * dim;
+  for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = e / dim;
+    const int c = (int)(e - r * dim);
+    out[e] = philox_entry(key_n, key_c, step, source, (uint64_t)(row0 + r), dim, c);
+  }
+}
+
 int cnfot_philox_rows(void* stream, uint64_t key, uint32_t step, int32_t source, int64_t global_rows, int64_t row0,
                       int64_t rows, int32_t dim, float* out) {
-  if (rows < 0 || row0 < 0 || row0 + rows > global_rows || dim < 1 || dim > kMaxDim)
-    return fail(CNFOT_ERR_ARG, "philox_rows: need 0 <= row0, row0 + rows <= global_rows, 1 <= dim <= %d", kMaxDim);
+  if (rows < 0 || row0 < 0 || row0 + rows > global_rows || dim < 1 || dim > kWideMaxDim)
+    return fail(CNFOT_ERR_ARG, "philox_rows: need 0 <= row0, row0 + rows <= global_rows, 1 <= dim <= %d", kWideMaxDim);
   if (source != CNFOT_ROWS_NORMAL && source != CNFOT_ROWS_OT_SOURCE) return fail(CNFOT_ERR_ARG, "philox_rows: unknown row source");
   if (rows == 0) return 0;
   if (!out) return fail(CNFOT_ERR_ARG, "NULL buffer");
-  int64_t blocks = (rows + 255) / 256;
+  const unsigned long long key_n = key ^ philox_salt(kDrawNormal, (uint64_t)global_rows);
+  const unsigned long long key_c = key ^ philox_salt(kDrawCategorical, (uint64_t)global_rows);
+  const int64_t work = dim <= kMaxDim ? rows : rows * dim;
+  int64_t blocks = (work + 255) / 256;
   if (blocks > 148 * 8) blocks = 148 * 8;
-  philox_rows_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(
-      key ^ philox_salt(kDrawNormal, (uint64_t)global_rows), key ^ philox_salt(kDrawCategorical, (uint64_t)global_rows), step,
-      source, row0, rows, dim, out);
+  if (dim <= kMaxDim)
+    philox_rows_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(key_n, key_c, step, source, row0, rows, dim, out);
+  else
+    philox_entries_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(key_n, key_c, step, source, row0, rows, dim, out);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return cuda_fail(e, "philox_rows_kernel launch");
   return 0;

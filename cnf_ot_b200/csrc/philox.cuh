@@ -171,7 +171,13 @@ CNFOT_PHILOX_HD float philox_entry(uint64_t key_n, uint64_t key_c, uint32_t step
       }
       v += c == 0 ? cx : cy;
     } else {
+#if defined(__CUDA_ARCH__)
+      // a separately rounded add, as philox_row computes it: contracted with z = r c into one FMA it would round once
+      // and differ from philox_row's number by up to one ulp in the kernels where the compiler fuses the two
+      v = __fadd_rn(v, -3.0f);
+#else
       v -= 3.0f;
+#endif
     }
   }
   return v;

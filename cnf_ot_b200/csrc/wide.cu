@@ -37,6 +37,7 @@ namespace {
 constexpr int kMaxM = 4;
 constexpr int kMaxPass = 5;   // flow passes alive at once: r(t-dt/2), r(t+dt/2), r(t), and the two shifted log-prob passes
 constexpr int kThreads = 256;
+constexpr int kInWgradSlice = 64;   // state columns per thread in wide_in_wgrad_kernel (KV4 <= 16 float4s)
 
 inline int round_up(int v, int m) { return (v + m - 1) / m * m; }
 inline int64_t round_up64(int64_t v, int64_t m) { return (v + m - 1) / m * m; }
@@ -49,7 +50,9 @@ struct WideDims {
 WideDims make_dims(const FlowLayout& lay) {
   WideDims w;
   w.D = lay.D; w.L = lay.L; w.M = lay.M; w.H = lay.H; w.Pp = lay.Pp;
-  w.Kx = round_up(lay.D + 1, 16);
+  // D <= 63: one slice of <= 64 columns in steps of 16.  Wider rows: whole 64-column slices, so that the transposed
+  // input GEMM (N = Kx) lands on the 64 / 128 / 256-wide dense_tc tiles and wide_in_wgrad_kernel walks 256-byte slices.
+  w.Kx = lay.D + 1 <= kInWgradSlice ? round_up(lay.D + 1, 16) : round_up(lay.D + 1, kInWgradSlice);
   w.prep_mlp = 2 * ((int64_t)w.Kx * w.H + (int64_t)(w.M - 1) * w.H * w.H + (int64_t)w.H * w.Pp);
   return w;
 }
@@ -486,14 +489,25 @@ constexpr size_t out_bwd_smem() { return (size_t)kRingStages * kRingRows * (kOut
 // Weight gradient of the input layer: dW0[w0_row(k)][h] += sum_r S[r][k] G1[r][h], db0[h] += sum_r G1[r][h];
 // a thread owns 2 hidden units (256 apart), 4 KV4 state columns accumulated in registers for each; G1 rows (the
 // CTA's 512 columns) and the state rows arrive through the bulk-copy ring.
+// SLICED (Kx > 64, KV4 = 16): blockIdx.z takes the state columns [64 z, 64 z + 64); the ring holds that 256-byte slice of
+// each row.  A slice the conditioner does not read at all (no column with a weight row) returns at once; db0 is summed
+// by the slice that holds the time column D.
 constexpr int kInWgradTH = 2;
 constexpr int kInWgradCols = kThreads * kInWgradTH;
-template <int KV4>
+template <int KV4, bool SLICED = false>
 __global__ void __launch_bounds__(kThreads)
 wide_in_wgrad_kernel(const float* __restrict__ S, int Kx, const float* __restrict__ G1, int64_t n, int H, int D, int d, int rev,
                      float* __restrict__ dW0, float* __restrict__ db0) {
   constexpr int KV = 4 * KV4, TH = kInWgradTH;
-  extern __shared__ __align__(128) float ring[];   // [stage][kRingRows][kInWgradCols] | [stage][kRingRows][Kx]
+  static_assert(!SLICED || KV == kInWgradSlice, "a sliced CTA owns one whole slice");
+  const int c0 = SLICED ? (int)blockIdx.z * kInWgradSlice : 0;
+  const int sw = SLICED ? kInWgradSlice : Kx;      // floats of a state row in the ring
+  if (SLICED) {
+    bool any = false;
+    for (int k = 0; k < KV; ++k) any |= w0_row(c0 + k, D, d, rev) >= 0;
+    if (!any) return;
+  }
+  extern __shared__ __align__(128) float ring[];   // [stage][kRingRows][kInWgradCols] | [stage][kRingRows][sw]
   __shared__ __align__(8) uint64_t full[kRingStages];
   float* ringG = ring;
   float* ringS = ring + kRingStages * kRingRows * kInWgradCols;
@@ -511,10 +525,15 @@ wide_in_wgrad_kernel(const float* __restrict__ S, int Kx, const float* __restric
     const int sidx = t % kRingStages;
     const int64_t r0 = lo + (int64_t)t * kRingRows;
     const int cnt = hi - r0 < kRingRows ? (int)(hi - r0) : kRingRows;
-    ring_expect(&full[sidx], (uint32_t)(cnt * (hcount + Kx) * 4));
+    ring_expect(&full[sidx], (uint32_t)(cnt * (hcount + sw) * 4));
     for (int rr = 0; rr < cnt; ++rr)
       ring_copy(ringG + (sidx * kRingRows + rr) * kInWgradCols, G1 + (r0 + rr) * H + hbase, (uint32_t)(hcount * 4), &full[sidx]);
-    ring_copy(ringS + sidx * kRingRows * Kx, S + r0 * Kx, (uint32_t)(cnt * Kx * 4), &full[sidx]);
+    if (SLICED) {
+      for (int rr = 0; rr < cnt; ++rr)
+        ring_copy(ringS + (sidx * kRingRows + rr) * sw, S + (r0 + rr) * Kx + c0, (uint32_t)(sw * 4), &full[sidx]);
+    } else {
+      ring_copy(ringS + sidx * kRingRows * Kx, S + r0 * Kx, (uint32_t)(cnt * Kx * 4), &full[sidx]);
+    }
   };
   if (tid == 0) {
     for (int q = 0; q < kRingStages; ++q) ring_init(&full[q]);
@@ -536,7 +555,7 @@ wide_in_wgrad_kernel(const float* __restrict__ S, int Kx, const float* __restric
     const int cnt = hi - r0 < kRingRows ? (int)(hi - r0) : kRingRows;
     ring_wait(&full[sidx], (uint32_t)((t / kRingStages) & 1));
     const float* tg = ringG + sidx * kRingRows * kInWgradCols + tid;
-    const float* ts = ringS + sidx * kRingRows * Kx;
+    const float* ts = ringS + sidx * kRingRows * sw;
 #pragma unroll 2
     for (int rr = 0; rr < cnt; ++rr) {
       float g[TH];
@@ -547,7 +566,7 @@ wide_in_wgrad_kernel(const float* __restrict__ S, int Kx, const float* __restric
       }
 #pragma unroll
       for (int q = 0; q < KV4; ++q) {
-        const float4 sv = *reinterpret_cast<const float4*>(ts + rr * Kx + 4 * q);
+        const float4 sv = *reinterpret_cast<const float4*>(ts + rr * sw + 4 * q);
 #pragma unroll
         for (int j = 0; j < TH; ++j) {
           acc[j][4 * q] += g[j] * sv.x; acc[j][4 * q + 1] += g[j] * sv.y;
@@ -564,13 +583,14 @@ wide_in_wgrad_kernel(const float* __restrict__ S, int Kx, const float* __restric
       const int h = h0 + kThreads * j;
 #pragma unroll
       for (int k = 0; k < KV; ++k) {
-        const int row = w0_row(k, D, d, rev);
+        const int row = w0_row(c0 + k, D, d, rev);
         if (row >= 0) asm volatile("red.global.add.f32 [%0], %1;" ::"l"(dW0 + (int64_t)row * H + h), "f"(acc[j][k]) : "memory");
       }
-      atomicAdd(db0 + h, bsum[j]);
+      if (!SLICED || (int)blockIdx.z == D / kInWgradSlice) atomicAdd(db0 + h, bsum[j]);
     }
 }
-inline size_t in_wgrad_smem(int Kx) { return (size_t)kRingStages * kRingRows * (kInWgradCols + Kx) * sizeof(float); }
+// sw: floats of a state row in the ring (Kx, or one 64-column slice)
+inline size_t in_wgrad_smem(int sw) { return (size_t)kRingStages * kRingRows * (kInWgradCols + sw) * sizeof(float); }
 
 // ---- loss heads ------------------------------------------------------------------------------------------
 __device__ __forceinline__ void block_add(double v, double* dst) {
@@ -632,10 +652,15 @@ wide_kinetic_head_kernel(const float* __restrict__ R1, const float* __restrict__
   if (R3) block_add(lp, slot_pot);
 }
 
-constexpr int kMaxWideDim = 64;
+// The per-row heads below hold D-float arrays in local memory; NX is their bound.  They are instantiated at 64 (every
+// dim up to 64) and at 256 (up to kWideMaxDim): the driver reserves local memory per resident thread for the largest
+// frame a launch needs, so the small dims keep their small frames.
+constexpr int kHeadSmall = 64, kHeadLarge = 256;
+static_assert(kWideMaxDim < kHeadLarge, "head arrays hold a whole row");
 
 // Rows pushed through the sample direction at time t (row_sample_terms of step_math.cuh):
 // do_fit: reverse_kl_loss_fn (applications.py:129-163)  w_fit (log p(y) - log q_t(y));  do_pot: potential_loss_fn (:176-205)
+template <int NX>
 __global__ void __launch_bounds__(kThreads)
 wide_sample_head_kernel(const float* __restrict__ Z0, const float* __restrict__ Y, const float* __restrict__ LD, int64_t n,
                         int D, int Kx, float t, int do_fit, int do_pot, StepConsts<float> pc, float* __restrict__ G,
@@ -643,7 +668,7 @@ wide_sample_head_kernel(const float* __restrict__ Z0, const float* __restrict__ 
   const int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   double lf = 0.0, lpot = 0.0;
   if (r < n) {
-    float y[kMaxWideDim], g[kMaxWideDim];
+    float y[NX], g[NX];
     float r2 = 0.f, z2 = 0.f;
     for (int c = 0; c < D; ++c) {
       y[c] = Y[r * Kx + c];
@@ -671,7 +696,7 @@ wide_sample_head_kernel(const float* __restrict__ Z0, const float* __restrict__ 
       for (int c = 0; c < D; ++c) g[c] += pc.w_fit * coef * y[c];
     }
     if (do_pot) {
-      float gp[kMaxWideDim];
+      float gp[NX];
       const float v = potential_value_grad<float>(pc.potential, pc.a, y, D, gp);
       lpot = (double)pc.w_pot * (double)v;
       for (int c = 0; c < D; ++c) g[c] += pc.w_pot * gp[c];
@@ -685,6 +710,7 @@ wide_sample_head_kernel(const float* __restrict__ Z0, const float* __restrict__ 
 // Coordinate i of kinetic_with_score_loss_fn / flow_matching_loss_fn (applications.py:245-374; row_kinetic of
 // step_math.cuh): score_i from the two shifted log-prob passes, resid_i = (r2_i - r1_i)/dt + kappa score_i - truth_i,
 // loss += w_kin resid_i^2; seeds the adjoints of the five passes.
+template <int NX>
 __global__ void __launch_bounds__(kThreads)
 wide_score_head_kernel(int i, const float* __restrict__ R1, const float* __restrict__ R2, const float* __restrict__ R3,
                        const float* __restrict__ Zp, const float* __restrict__ LDp, const float* __restrict__ Zm,
@@ -703,7 +729,7 @@ wide_score_head_kernel(int i, const float* __restrict__ R1, const float* __restr
     const float score = ((-0.5f * zp2 + LDp[r]) - (-0.5f * zm2 + LDm[r])) / pc.dx;
     float truth_i = 0.f;
     if (pc.type == kFP) {
-      float r3[kMaxWideDim], truth[kMaxWideDim];
+      float r3[NX], truth[NX];
       for (int c = 0; c < D; ++c) { r3[c] = R3[r * Kx + c]; truth[c] = 0.f; }
       drift_value<float>(pc.drift, pc.a, r3, D, truth);
       truth_i = truth[i];
@@ -733,12 +759,13 @@ wide_add2_kernel(float* __restrict__ G3, const float* __restrict__ Gp, const flo
 }
 
 // fp: resid = v - truth(r3): pull the residual adjoints back through the drift target (applications.py:308-372)
+template <int NX>
 __global__ void __launch_bounds__(kThreads)
 wide_drift_pullback_kernel(const float* __restrict__ R3, const float* __restrict__ GRES, int64_t n, int D, int Kx,
                            StepConsts<float> pc, float* __restrict__ G3) {
   const int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (r >= n) return;
-  float r3[kMaxWideDim], gres[kMaxWideDim], g3[kMaxWideDim];
+  float r3[NX], gres[NX], g3[NX];
   for (int c = 0; c < D; ++c) { r3[c] = R3[r * Kx + c]; gres[c] = GRES[r * Kx + c]; g3[c] = G3[r * Kx + c]; }
   drift_pullback<float>(pc.drift, pc.a, r3, D, gres, g3);
   for (int c = 0; c < D; ++c) G3[r * Kx + c] = g3[c];
@@ -884,6 +911,7 @@ wide_init_shift_kernel(const float* __restrict__ R3, int64_t n, int D, int Kx, i
 // All coordinates of the score-kinetic term at once (wide_score_head_kernel for every i): Z / LD hold the 2 D n
 // latent outputs / log-dets of the shifted log-prob passes; seeds Gs (2 D n rows), GLs, the adjoints of r1, r2
 // (G1, G2; every column written), zeroes G3 and fills GRES.
+template <int NX>
 __global__ void __launch_bounds__(kThreads)
 wide_score_head_all_kernel(const float* __restrict__ R1, const float* __restrict__ R2, const float* __restrict__ R3,
                            const float* __restrict__ Z, const float* __restrict__ LDs, int64_t n, int D, int Kx,
@@ -893,10 +921,10 @@ wide_score_head_all_kernel(const float* __restrict__ R1, const float* __restrict
   const int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   double lk = 0.0;
   if (r < n) {
-    float truth[kMaxWideDim];
+    float truth[NX];
     for (int c = 0; c < D; ++c) truth[c] = 0.f;
     if (pc.type == kFP) {
-      float r3[kMaxWideDim];
+      float r3[NX];
       for (int c = 0; c < D; ++c) r3[c] = R3[r * Kx + c];
       drift_value<float>(pc.drift, pc.a, r3, D, truth);
     }
@@ -1037,6 +1065,10 @@ wide_vjp_out_kernel(const float* __restrict__ G, const float* __restrict__ g_log
   }
 }
 
+// the instantiation of a per-row head for rows of D coordinates
+template <typename F>
+F head_for(int D, F small, F large) { return D <= kHeadSmall ? small : large; }
+
 // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) only when a (kernel, device) needs more than it was given before:
 // the call costs microseconds, a small-batch step makes hundreds of launches
 cudaError_t set_smem_max(const void* kern, size_t bytes, int (&cur)[64]) {
@@ -1176,14 +1208,22 @@ struct WideEngine {
     }
     if (!ok()) return;
     // input layer: dW0 / db0 on CUDA cores, the input adjoints accumulated into the adjoint state by the GEMM epilogue
-    const int kv4 = (wd.D + 1 + 3) / 4;
+    const bool sliced = Kx > kInWgradSlice;
+    const int kv4 = sliced ? kInWgradSlice / 4 : (wd.D + 1 + 3) / 4;
+    const int nz = sliced ? Kx / kInWgradSlice : 1;
     const int hb = (H + kInWgradCols - 1) / kInWgradCols;
     int64_t ny = (n + 63) / 64;
-    if (ny * hb > 296) ny = 296 / hb;
+    if (ny * hb * nz > 296) ny = 296 / (hb * nz);
     if (ny < 1) ny = 1;
-    dim3 grid((unsigned)hb, (unsigned)ny);
-    const size_t ring_bytes = in_wgrad_smem(Kx);
-    switch (kv4) {
+    dim3 grid((unsigned)hb, (unsigned)ny, (unsigned)nz);
+    const size_t ring_bytes = in_wgrad_smem(sliced ? kInWgradSlice : Kx);
+    if (sliced) {
+      static int cur[64] = {};
+      check(set_smem_max((const void*)wide_in_wgrad_kernel<kInWgradSlice / 4, true>, ring_bytes, cur), "cudaFuncSetAttribute");
+      if (!ok()) return;
+      wide_in_wgrad_kernel<kInWgradSlice / 4, true><<<grid, kThreads, ring_bytes, s>>>(cst, Kx, gc, n, H, wd.D, d, layer & 1,
+                                                                                     grad + off_w0, grad + off_b0);
+    } else switch (kv4) {
 #define CNFOT_IN_WGRAD(Q)                                                                                              \
   case Q: {                                                                                                            \
     static int cur[64] = {};                                                                                           \
@@ -1430,7 +1470,8 @@ void kinetic_chunk(WideEngine& e, const StepConsts<float>& pc, const PassSrc& rt
       e.flow_pass<K>(1, 3, n);
       e.flow_pass<K>(1, 4, n);
       if (!e.ok()) return;
-      wide_score_head_kernel<<<WideEngine::blocks_for(n), kThreads, 0, e.s>>>(
+      const auto score_head = head_for(D, wide_score_head_kernel<kHeadSmall>, wide_score_head_kernel<kHeadLarge>);
+      score_head<<<WideEngine::blocks_for(n), kThreads, 0, e.s>>>(
           i, e.state(0, L), e.state(1, L), e.state(2, L), e.state(3, L), e.LD[3], e.state(4, L), e.LD[4], n, D, Kx, pc, e.G[0],
           e.G[1], e.G[3], e.G[4], e.GL, e.GL2, e.GRES, e.slots + kSlotKinetic);
       e.check_launch("wide_score_head_kernel launch");
@@ -1441,7 +1482,8 @@ void kinetic_chunk(WideEngine& e, const StepConsts<float>& pc, const PassSrc& rt
       e.check_launch("wide_add2_kernel launch");
     }
     if (pc.type == kFP && e.ok()) {
-      wide_drift_pullback_kernel<<<WideEngine::blocks_for(n), kThreads, 0, e.s>>>(e.state(2, L), e.GRES, n, D, Kx, pc, e.G[2]);
+      const auto pullback = head_for(D, wide_drift_pullback_kernel<kHeadSmall>, wide_drift_pullback_kernel<kHeadLarge>);
+      pullback<<<WideEngine::blocks_for(n), kThreads, 0, e.s>>>(e.state(2, L), e.GRES, n, D, Kx, pc, e.G[2]);
       e.check_launch("wide_drift_pullback_kernel launch");
     }
   }
@@ -1482,7 +1524,8 @@ void kinetic_chunk_batched(WideEngine& e, const StepConsts<float>& pc, const Pas
     e.init_shift(1, r1 + 2 * blk, n, pc.dx / 2.f);
     e.flow_pass<K>(1, 1, n * 2 * D);
     if (!e.ok()) return;
-    wide_score_head_all_kernel<<<WideEngine::blocks_for(n), kThreads, 0, e.s>>>(
+    const auto score_head_all = head_for(D, wide_score_head_all_kernel<kHeadSmall>, wide_score_head_all_kernel<kHeadLarge>);
+    score_head_all<<<WideEngine::blocks_for(n), kThreads, 0, e.s>>>(
         r1, r1 + blk, r1 + 2 * blk, e.state(1, L), e.LD[1], n, D, Kx, pc, g1, g1 + blk, g1 + 2 * blk, e.G[1], e.GL, e.GRES,
         e.slots + kSlotKinetic);
     e.check_launch("wide_score_head_all_kernel launch");
@@ -1491,7 +1534,8 @@ void kinetic_chunk_batched(WideEngine& e, const StepConsts<float>& pc, const Pas
     wide_fold_kernel<<<WideEngine::grid_for(blk), kThreads, 0, e.s>>>(g1 + 2 * blk, e.G[1], n, 2 * D, Kx);
     e.check_launch("wide_fold_kernel launch");
     if (pc.type == kFP) {
-      wide_drift_pullback_kernel<<<WideEngine::blocks_for(n), kThreads, 0, e.s>>>(r1 + 2 * blk, e.GRES, n, D, Kx, pc, g1 + 2 * blk);
+      const auto pullback = head_for(D, wide_drift_pullback_kernel<kHeadSmall>, wide_drift_pullback_kernel<kHeadLarge>);
+      pullback<<<WideEngine::blocks_for(n), kThreads, 0, e.s>>>(r1 + 2 * blk, e.GRES, n, D, Kx, pc, g1 + 2 * blk);
       e.check_launch("wide_drift_pullback_kernel launch");
     }
   }
@@ -1588,7 +1632,8 @@ void run_step(WideEngine& e, const StepConsts<float>& pc, const StepRows& in, in
       e.flow_pass<K>(0, 0, 2 * n, true);
       if (!e.ok()) break;
       for (int seg = 0; seg < 2; ++seg) {
-        wide_sample_head_kernel<<<WideEngine::blocks_for(n), kThreads, 0, e.s>>>(
+        const auto sample_head = head_for(D, wide_sample_head_kernel<kHeadSmall>, wide_sample_head_kernel<kHeadLarge>);
+        sample_head<<<WideEngine::blocks_for(n), kThreads, 0, e.s>>>(
             e.state(0, 0) + seg * n * Kx, e.state(0, L) + seg * n * Kx, e.LD[0] + seg * n, n, D, Kx, seg == 0 ? 0.f : pc.horizon, seg == 0,
             seg == 1, pc, e.G[0] + seg * n * Kx, e.slots + kSlotFit0, e.slots + kSlotPotential);
         e.check_launch("wide_sample_head_kernel launch");
@@ -1607,7 +1652,8 @@ void run_step(WideEngine& e, const StepConsts<float>& pc, const StepRows& in, in
       e.init_states(0, in.at(in.latent, kRowsNormal, false, r0, t), n);
       e.flow_pass<K>(0, 0, n, true);
       if (!e.ok()) break;
-      wide_sample_head_kernel<<<WideEngine::blocks_for(n), kThreads, 0, e.s>>>(
+      const auto sample_head = head_for(D, wide_sample_head_kernel<kHeadSmall>, wide_sample_head_kernel<kHeadLarge>);
+      sample_head<<<WideEngine::blocks_for(n), kThreads, 0, e.s>>>(
           e.state(0, 0), e.state(0, L), e.LD[0], n, D, Kx, t, do_fit, do_pot, pc, e.G[0], e.slots + kSlotFit0,
           e.slots + kSlotPotential);
       e.check_launch("wide_sample_head_kernel launch");
@@ -1618,13 +1664,21 @@ void run_step(WideEngine& e, const StepConsts<float>& pc, const StepRows& in, in
 
 }  // namespace
 
+static_assert(kWideMaxDim == 255, "wide_supported's message names the bound");
 bool wide_supported(const FlowLayout& lay, const char** why) {
   const char* w = nullptr;
   if (lay.D < 2) w = "wide engine needs dim >= 2";
   else if (lay.H < 16 || lay.H % 16 || (lay.H > 64 && lay.H % 64)) w = "wide engine needs hidden in {16, 32, 48} or a multiple of 64";
   else if (lay.M < 1 || lay.M > kMaxM) w = "wide engine supports 1..4 hidden layers";
   else if (lay.K != 5) w = "wide engine is instantiated for num_bins == 5";
-  else if (lay.D + 1 > 64) w = "wide engine supports dim <= 63";
+  else if (lay.D > kWideMaxDim) w = "wide engine supports dim <= 255";
+  else if ((int64_t)lay.L * (lay.D - 1) > 65535) w = "wide engine needs num_layers * (dim - 1) <= 65535";
+  if (!w) {
+    // FlowLayout offsets are int: the whole blob must stay below 2^31 floats (make_layout's sums, in 64 bits)
+    const int64_t H = lay.H, mlp_const = H + (lay.M - 1) * (H * H + H) + H * lay.Pp + lay.Pp;
+    const int64_t layer_stride = (int64_t)(lay.D - 1) * mlp_const + H * ((int64_t)(lay.D - 1) * (lay.D + 2) / 2);
+    if (lay.Pp + lay.L * layer_stride > INT32_MAX) w = "wide engine needs a parameter blob below 2^31 floats";
+  }
   if (why) *why = w;
   return w == nullptr;
 }

@@ -11,6 +11,10 @@
 
 namespace cnfot {
 
+// Largest dim the engine takes: a state row [x | t | 0 ..] is then at most 256 columns, one N = 256 tile of the
+// input-adjoint GEMM.  cnfot_philox_rows draws rows of every dim up to this bound.
+constexpr int kWideMaxDim = 255;
+
 bool wide_supported(const FlowLayout& lay, const char** why);
 // workspace: prepared weights (2 x 2 x every matrix) + the chunk buffers
 int64_t wide_step_workspace_bytes(const FlowLayout& lay, int64_t rows_B, int64_t rows_b);

@@ -259,7 +259,8 @@ CNFOT_API int cnfot_mfc_step_dp(void* stream, const cnfot_flow_desc* flow, const
  * generates its rows itself (nothing crosses PCIe or HBM) and any shard is generated independently of how
  * the batch is split over GPUs.  jax.random's threefry streams are not reproduced.
  *   cnfot_philox_rows        rows [row0, row0 + rows) of the (global_rows, dim) array of that draw, as an array:
- *                            feed the explicit-input entries or a CPU check
+ *                            feed the explicit-input entries or a CPU check; 1 <= dim <= 255 (the widest flow
+ *                            the wide-conditioner engine runs)
  *   cnfot_philox_times_host  the n_t uniform times horizon * U[0,1) of a step, computed on the host
  *   cnfot_mfc_step_rng       cnfot_mfc_step[_dp] (peers may be NULL) with the draws made inside the kernel:
  *                            latent / target rows = NORMAL (global_B, dim), source rows = OT_SOURCE (global_B, dim),
